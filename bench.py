@@ -47,7 +47,15 @@ def parse_args():
     ap.add_argument("--reads", type=int, default=10000, help="reads per GPU")
     ap.add_argument("--events", type=int, default=4000, help="events per read")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the per-job scores of the last step to DIR/scores.npy (float32, job order; "
+                         "every rank's jobs in rank order at --gpus N), so that two builds can be compared on identical inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "scorereads" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the default workload (--workload scorereads, --impl ours)")
+    return args
 
 
 def peaks():
@@ -414,7 +422,7 @@ def call_methylation_block(args, rank, world, local, steps, warmup):
     for _ in range(2):
         tsv_bytes = e2e_step()
     barrier()
-    e2e_steps = max(3, min(steps, 10))
+    e2e_steps = steps
     stage = np.zeros(2)
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
@@ -598,7 +606,7 @@ def variants_block(args, rank, world, local, steps, warmup):
     for _ in range(2):
         e2e_step()
     barrier()
-    e2e_steps = max(3, min(steps, 10))
+    e2e_steps = steps
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
         q2, nr2, _ = e2e_step()
@@ -936,6 +944,13 @@ def run_aux(args, rank, world, local, saved_stdout):
     eng.close()
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """DIR/<name>.npy of each device tensor, as the caller of the timed path receives it"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def emit(line: dict, saved_stdout: int) -> None:
     """Exactly one JSON line on the real stdout (libraries such as NCCL print banners to fd 1)."""
     sys.stdout.flush()
@@ -1038,9 +1053,10 @@ def main():
     from nanopolish_b200.dist import gather_to_rank0
 
     def step():
+        nonlocal gathered
         eng.hmm_score(scores.data_ptr())
         if world > 1:
-            gather_to_rank0(scores, counts)           # one NCCL gather of per-job log-likelihoods over NVLink
+            gathered = gather_to_rank0(scores, counts)           # one NCCL gather of per-job log-likelihoods over NVLink
 
     def barrier():
         if world > 1:
@@ -1068,6 +1084,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"scores": torch.cat(gathered) if world > 1 else scores[:n_jobs]})
 
     # kernel-only duration for the roofline: CUDA events around each kernel sequence, on its stream
     for _ in range(5):
@@ -1091,7 +1109,7 @@ def main():
         e2e_step()
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         e2e_step()
     torch.cuda.synchronize()
@@ -1142,7 +1160,7 @@ def main():
     cm = None
     if not args.no_call_methylation:
         try:
-            cm = call_methylation_block(args, rank, world, local, max(3, min(args.steps, 10)), args.warmup)
+            cm = call_methylation_block(args, rank, world, local, args.steps, args.warmup)
         except Exception as ex:          # never lose the headline line over the extra block
             cm = {"error": f"{type(ex).__name__}: {ex}"} if rank == 0 else None
     if rank == 0:

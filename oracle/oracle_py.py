@@ -402,5 +402,9 @@ class RefOracle:
         self.lib.npref_logsum_table(_p(t))
         return t
 
+    def add_logs(self, a, b):
+        """add_logs(a[i], b[i]) for each i, as float32"""
+        return np.array([self.lib.npref_add_logs(float(x), float(y)) for x, y in zip(a, b)], np.float32)
+
     def max_threads(self):
         return int(self.lib.npref_max_threads())

@@ -19,11 +19,25 @@ def port_oracle():
 
 
 @pytest.fixture(scope="session")
-def ref_oracle():
+def _compiled_ref():
     from oracle.oracle_py import RefOracle
-    if not RefOracle.available():
-        pytest.skip("compiled reference (oracle/_ref/libnpref.so) not present on this box")
-    return RefOracle()
+    return RefOracle() if RefOracle.available() else None
+
+
+@pytest.fixture
+def ref_oracle(request, _compiled_ref):
+    """The compiled reference (oracle/_ref/libnpref.so) where it is built; elsewhere its answers recorded under
+    tests/golden/ref_calls/ (tests/ref_replay.py).  NPH_RECORD_REF=<dir> records them from the compiled reference into <dir>."""
+    from tests.ref_replay import ReplayedRef
+    record_dir = os.environ.get("NPH_RECORD_REF")
+    if record_dir and _compiled_ref is None:
+        pytest.fail("NPH_RECORD_REF is set but the compiled reference (oracle/_ref/libnpref.so) is not built")
+    if _compiled_ref is not None and not record_dir:
+        yield _compiled_ref
+        return
+    ref = ReplayedRef(request.node, _compiled_ref, record_dir)
+    yield ref
+    ref.finish()
 
 
 @pytest.fixture(scope="session")

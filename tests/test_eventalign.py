@@ -3,7 +3,7 @@
 TSV / SAM / summary writers).
 
   * the Python restatement (oracle/eventalign_py.py) against the COMPILED reference's align_read_to_ref +
-    emit_event_alignment_tsv (oracle/_ref, where /root/reference exists) and against the outputs recorded from it
+    emit_event_alignment_tsv (oracle/_ref, or its answers recorded under tests/golden/ref_calls/) and against the outputs recorded from it
     (tests/golden/eventalign_golden.npz) anywhere;
   * the C++ cursor logic on the CPU: rounds are pulled out of EventAligner, the paths come from the plain-C Viterbi
     oracle and are fed back — the text it then writes must equal the reference's, byte for byte;

@@ -169,7 +169,8 @@ def test_invalid_inputs(eng2):
 
 def test_device_equals_compiled_reference(eng2, ref_oracle):
     """nph_methylation_batch against the compiled reference's own calculate_methylation_for_read + TSV writer (oracle/_ref,
-    which travels to the GPU box): records built the way BAM / FASTA / SquiggleRead present them (tests/meth_cases.py)."""
+    or its answers recorded under tests/golden/ref_calls/): records built the way BAM / FASTA / SquiggleRead present them
+    (tests/meth_cases.py)."""
     from tests import meth_cases as mc
     nuc = synth.load_model("nucleotide")
     rs = synth.gen_reads(9, 2200, nuc, seed=4242, cpg_keep=0.35)
