@@ -587,6 +587,50 @@ int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_samples_tot
  * --samples / --signal-index read back.  NPH_ERR_STATE if n_jobs is not that call's job count. */
 int nph_last_trim_ranges(nph_ctx* ctx, nph_raw_range* ranges_out, size_t n_jobs);
 
+/* ---- poly(A) tail length of direct-RNA reads (section 8f N5: `nanopolish polya`) -------------------------------
+ * Per read, what estimate_polya_for_single_read computes once load_from_raw has run (ref:
+ * src/nanopolish_polya_estimator.cpp): SegmentationHMM's 6-state Viterbi over every trimmed raw sample (:204-509) with the
+ * Gaussians scaled by the read's (float) scale / shift / var, segment_squiggle's region ends and cliff count,
+ * estimate_unaligned_duration_profile's read rate (:564-599), estimate_polya_length (:638-662) and the two QC verdicts
+ * that need no alignment record: post_segmentation_qc (NOREGION) and post_estimation_qc (ADAPTER).  SUFFCLIP comes from
+ * the BAM record's last CIGAR op and is the caller's (nph::PolyaEstimator in nanopolish_b200/host/nph_polya.hpp).
+ * Emissions use glibc's expf / logf restated bit for bit (csrc/polya_math.cuh), so results equal the reference's on an
+ * x86-64 host with glibc >= 2.28. */
+typedef struct {
+    uint64_t sample_off;      /* first trimmed raw sample of the read in samples[] (acquisition order, picoamps) */
+    uint64_t event_off;       /* first event duration in durations[] (the read's events in SquiggleRead order) */
+    uint64_t map_off;         /* first base_to_event_map entry of the read in map[] (event indices relative to event_off) */
+    uint32_t n_samples;       /* >= 2 */
+    uint32_t n_events;        /* 0: the read did not load (READ_FAILED_LOAD); nothing else of the job is read */
+    uint32_t n_kmers;         /* read_sequence.length() - k + 1 map entries, >= 1 */
+    uint32_t reserved;
+    double sample_rate;
+    double shift, scale, var; /* sr.scalings[0] */
+} nph_polya_job;              /* 72 bytes */
+#define NPH_POLYA_NOREGION     1   /* fewer than 200 adapter or poly(A) samples */
+#define NPH_POLYA_ADAPTER      2   /* more than 300 adapter nucleotides */
+#define NPH_POLYA_FAILED_LOAD  4   /* no events: no other field is set */
+typedef struct {
+    uint64_t start, leader, adapter, polya;   /* Segmentation: last sample index of S, L, A and P/C (size_t arithmetic) */
+    uint64_t cliffs;                          /* samples in state C */
+    double read_rate;                         /* 1 / median per-k-mer duration */
+    double polya_length;                      /* nucleotides, >= 0 */
+    float end_score;                          /* viterbi_scores[n_samples-1][TRANSCRIPT] */
+    uint32_t qc;                              /* NPH_POLYA_* bits */
+} nph_polya_result;           /* 64 bytes */
+/* One call: host buffers in, results out.  Jobs may share samples, durations and map entries.  A job with n_samples < 2, a sample / event / map range outside its buffer,
+ * no map entries, or a map entry outside [0, n_events) (start -1 means "no events" and is skipped) yields NPH_ERR_INVALID. */
+int nph_polya_batch(nph_ctx* ctx, const float* samples, size_t n_samples_total, const float* durations, size_t n_events_total,
+                    const nph_event_range* map, size_t n_map_total, const nph_polya_job* jobs, size_t n_jobs,
+                    nph_polya_result* results_out);
+/* The same over the reads of the most recent nph_load_from_raw_batch on this context, from what it left in device memory:
+ * the raw samples with their trim ranges, the event durations, the base_to_event_map, the calibrated scalings and the
+ * sample rates.  Nothing is uploaded.  A read whose calibration status is non-zero gets NPH_POLYA_FAILED_LOAD.  (For this,
+ * nph_load_from_raw_batch keeps the batch's raw samples on the device, 4 bytes per sample, until the next such call or
+ * nph_destroy.)
+ * NPH_ERR_STATE if n_jobs is not that call's job count, or if another call has reused its buffers since. */
+int nph_polya_after_load(nph_ctx* ctx, nph_polya_result* results_out, size_t n_jobs);
+
 /* ---- measurement hooks (used by bench.py; not part of the reference surface) ------------- */
 /* Device time in ms of the most recent nph_hmm_score / nph_abea_run kernel sequence, measured
  * with CUDA events on the context's stream (valid after a sync), and the number of kernel

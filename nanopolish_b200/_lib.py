@@ -75,6 +75,8 @@ def load() -> C.CDLL:
     lib.nph_screen_run.argtypes = [vp]
     lib.nph_screen_counts.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.nph_screen_fetch.argtypes = [vp, vp, vp, vp]
+    lib.nph_polya_batch.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, sz, vp]
+    lib.nph_polya_after_load.argtypes = [vp, vp, sz]
     lib.nph_last_kernel_ms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_int)]
     lib.nph_host_alloc.argtypes = [C.POINTER(vp), sz]
     lib.nph_host_free.argtypes = [vp]
@@ -87,5 +89,5 @@ EXPORTS = [
     "nph_sync", "nph_stream", "nph_model_upload", "nph_hmm_score_batch", "nph_hmm_score_batch_seq", "nph_hmm_jobs_load_seq", "nph_reads_load",
     "nph_hmm_jobs_load", "nph_hmm_score", "nph_hmm_scores_fetch", "nph_score_set_combine",
     "nph_abea_batch", "nph_abea_jobs_load", "nph_abea_run", "nph_abea_fetch", "nph_mom_batch",
-    "nph_hmm_align_batch", "nph_hmm_align", "nph_eventalign_chain", "nph_detect_events_batch", "nph_trim_raw_batch", "nph_recalibrate_batch", "nph_load_from_raw_batch", "nph_last_trim_ranges", "nph_methylation_batch", "nph_methylation_batch_compact", "nph_methylation_load", "nph_methylation_load_compact", "nph_methylation_run", "nph_methylation_counts", "nph_methylation_fetch", "nph_methylation_sites_dev", "nph_methylation_tsv", "nph_methylation_batch_compact_tsv", "nph_screen_edits_batch", "nph_screen_load", "nph_screen_run", "nph_screen_counts", "nph_screen_fetch", "nph_last_kernel_ms", "nph_host_alloc", "nph_host_free",
+    "nph_hmm_align_batch", "nph_hmm_align", "nph_eventalign_chain", "nph_detect_events_batch", "nph_trim_raw_batch", "nph_recalibrate_batch", "nph_load_from_raw_batch", "nph_last_trim_ranges", "nph_methylation_batch", "nph_methylation_batch_compact", "nph_methylation_load", "nph_methylation_load_compact", "nph_methylation_run", "nph_methylation_counts", "nph_methylation_fetch", "nph_methylation_sites_dev", "nph_methylation_tsv", "nph_methylation_batch_compact_tsv", "nph_screen_edits_batch", "nph_screen_load", "nph_screen_run", "nph_screen_counts", "nph_screen_fetch", "nph_polya_batch", "nph_polya_after_load", "nph_last_kernel_ms", "nph_host_alloc", "nph_host_free",
 ]

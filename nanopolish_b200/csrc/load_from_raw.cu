@@ -127,9 +127,13 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     const size_t b_trim = nph_trim_scratch_bytes(rr.data(), n_jobs, 100);
     const size_t b_ed = nph_ed_scratch_bytes(n_samples_total, n_jobs, cap_total);
     const size_t b_small = al256(sizeof(uint64_t) * n_jobs) * 2 + al256(sizeof(uint32_t) * n_jobs) + al256(sizeof(double) * n_jobs);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, b_raw + std::max(b_trim, b_ed + b_small)));
-    float* d_raw = reinterpret_cast<float*>(ctx->d_abea_scratch.p);
-    uint8_t* arena = ctx->d_abea_scratch.p + b_raw;
+    // the samples get a buffer of their own so that they outlive the call (nph_polya_after_load reads them)
+    nph_ctx::LoadedRaw& kept = ctx->loaded_raw;
+    kept.valid = false;
+    NPH_TRY(nph_reserve(ctx, kept.d_raw, std::max<size_t>(b_raw / sizeof(float), 1)));
+    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, std::max(b_trim, b_ed + b_small)));
+    float* d_raw = kept.d_raw.p;
+    uint8_t* arena = ctx->d_abea_scratch.p;
     NPH_CUDA(ctx, cudaMemcpyAsync(d_raw, raw, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     int launches = 0;
@@ -150,9 +154,16 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     }
     std::vector<uint32_t> live;
     for (size_t j = 0; j < n_jobs; ++j) if (range[j].end > range[j].start) live.push_back((uint32_t)j);
+    kept.jobs.assign(jobs, jobs + n_jobs);
+    kept.live_index.assign(n_jobs, -1);
+    for (size_t t = 0; t < live.size(); ++t) kept.live_index[live[t]] = (int64_t)t;
+    kept.n_samples_total = n_samples_total; kept.n_ranks_total = n_ranks_total;
+    kept.d_duration = nullptr; kept.d_b2e = nullptr; kept.d_cal = nullptr;
     if (live.empty()) {
         if (base_to_event_out) for (size_t i = 0; i < n_ranks_total; ++i) base_to_event_out[i] = nph_event_range{-1, -1};
         for (size_t j = 0; j <= n_jobs; ++j) event_off_out[j] = 0;
+        kept.event_off.assign(n_jobs + 1, 0);
+        kept.valid = true;
         ctx->last_launches = launches; ctx->staged_ms = staged_ms; ctx->timing_valid = 2;
         return NPH_OK;
     }
@@ -277,6 +288,9 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
         NPH_CUDA(ctx, cudaMemcpyAsync(base_to_event_out, d_b2e, sizeof(nph_event_range) * n_ranks_total, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     for (size_t t = 0; t < nl; ++t) calibrations_out[live[t]] = cal[t];
+    kept.event_off.assign(event_off_out, event_off_out + n_jobs + 1);
+    kept.d_duration = d_dur; kept.d_b2e = d_b2e; kept.d_cal = d_cal;
+    kept.valid = true;
     NPH_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1)); staged_ms += ms;     // ev0 was recorded at the ABEA launch
     if (verbose) fprintf(stderr, "  abea+calibration %.2f ms  (total %.2f ms, %zu of %zu reads aligned)\n", ms, staged_ms, nl, n_jobs);
     ctx->last_launches = launches;

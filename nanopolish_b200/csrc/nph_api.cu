@@ -204,6 +204,7 @@ int nph_destroy(nph_ctx* ctx)
     free_buf(ctx->d_jobs); free_buf(ctx->d_trans); free_buf(ctx->d_order); free_buf(ctx->d_scores);
     free_buf(ctx->d_counters); free_buf(ctx->d_sched_cls); free_buf(ctx->d_sched_bkt); free_buf(ctx->d_sched_hist); free_buf(ctx->d_scratch); free_buf(ctx->d_abea_jobs); free_buf(ctx->d_abea_ranks);
     free_buf(ctx->d_pairs); free_buf(ctx->d_abea_res); free_buf(ctx->d_abea_scratch); free_buf(ctx->d_abea_order); free_buf(ctx->d_abea_consts); free_buf(ctx->d_prep);
+    free_buf(ctx->loaded_raw.d_raw); free_buf(ctx->d_polya);
     free_buf(ctx->meth.d_ref); free_buf(ctx->meth.d_pairs); free_buf(ctx->meth.d_records); free_buf(ctx->meth.d_prov_off); free_buf(ctx->meth.d_prov);
     free_buf(ctx->meth.d_counts); free_buf(ctx->meth.d_sites); free_buf(ctx->meth.d_tsv_in); free_buf(ctx->meth.d_tsv_off); free_buf(ctx->meth.d_tsv); free_buf(ctx->meth.d_deltas); free_buf(ctx->meth.d_dense);
     free_buf(ctx->screen.d_ref); free_buf(ctx->screen.d_deltas); free_buf(ctx->screen.d_dense); free_buf(ctx->screen.d_records);

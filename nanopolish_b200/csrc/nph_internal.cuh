@@ -174,6 +174,21 @@ struct nph_ctx {
     std::vector<float2> h_stage_trans;
     std::vector<nph_raw_range> h_last_trim;  // surviving sample range per job of the last nph_load_from_raw_batch
 
+    // what the last nph_load_from_raw_batch leaves for nph_polya_after_load (polya.cu): the raw samples in their own buffer,
+    // the compact event durations, the event map and the calibrations in d_prep (valid until d_prep is reused)
+    struct LoadedRaw {
+        bool valid = false;
+        DevBuf<float> d_raw;                 // every raw sample of the call, as uploaded
+        const float* d_duration = nullptr;   // compact job order over the live reads
+        const nph_event_range* d_b2e = nullptr;
+        const nph_calibration* d_cal = nullptr;   // live-read order
+        std::vector<nph_raw_job> jobs;
+        std::vector<int64_t> live_index;     // per job: index among the live reads, -1 if nothing survived the trim
+        std::vector<uint64_t> event_off;     // per job: first event in the compact layout (n_jobs + 1)
+        size_t n_samples_total = 0, n_ranks_total = 0;
+    } loaded_raw;
+    DevBuf<uint8_t> d_polya;                 // polya.cu: jobs, results, backpointers, per-k-mer durations (+ inputs of the one-shot call)
+
 };
 
 int nph_set_cuda_error(nph_ctx* ctx, cudaError_t e, const char* what);

@@ -522,6 +522,7 @@ extern "C" int nph_screen_fetch(nph_ctx* ctx, double* qualities_out, uint32_t* n
     const uint32_t n_pos = (uint32_t)m.n_pos;
     // outputs staged in the (now idle) score buffer region: 9 doubles + 1 uint32 per position
     DevBuf<uint8_t>& scratch = ctx->d_prep;
+    ctx->loaded_raw.valid = false;              // d_prep held the last load_from_raw batch's durations and map
     const size_t b_q = sizeof(double) * NPH_SCREEN_SLOTS * (size_t)n_pos, b_n = sizeof(uint32_t) * (size_t)n_pos;
     const size_t b_r = sizeof(unsigned long long) * (size_t)n_pos;
     NPH_TRY(nph_reserve(ctx, scratch, b_q + b_r + b_n + 256));

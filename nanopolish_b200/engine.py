@@ -344,6 +344,23 @@ class Engine:
         tot = int(off[-1])
         return off, mean[:tot], stdv[:tot], start[:tot], dur[:tot], b2e, cal
 
+    # ---- poly(A) tail length (nanopolish polya) -------------------------------------------------
+    def polya_batch(self, samples, durations, emap, jobs, out=None):
+        """== the device part of estimate_polya_for_single_read per POLYA_JOB_DT job: POLYA_RES_DT[n_jobs] (segmentation, cliffs,
+        read rate, tail length, Viterbi end score, NOREGION / ADAPTER / failed-load bits).  out: a (page-locked) result buffer."""
+        from .synth import POLYA_RES_DT
+        res = out if out is not None else np.zeros(jobs.shape[0], POLYA_RES_DT)
+        self._check(self.lib.nph_polya_batch(self.ctx, _p(samples), samples.shape[0], _p(durations), durations.shape[0], _p(emap),
+                                             emap.shape[0], _p(jobs), jobs.shape[0], _p(res)), "nph_polya_batch")
+        return res
+
+    def polya_after_load(self, n_jobs: int, out=None):
+        """polya over the reads of the last load_from_raw_batch, from what it left on the device (nothing is uploaded)."""
+        from .synth import POLYA_RES_DT
+        res = out if out is not None else np.zeros(n_jobs, POLYA_RES_DT)
+        self._check(self.lib.nph_polya_after_load(self.ctx, _p(res), n_jobs), "nph_polya_after_load")
+        return res
+
     # ---- measurement ----------------------------------------------------------------------
     def last_trim_ranges(self, n_jobs: int) -> np.ndarray:
         """[start, end) of the samples each job of the last load_from_raw_batch kept (what SRF_LOAD_RAW_SAMPLES stores)."""

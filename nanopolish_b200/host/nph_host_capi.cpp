@@ -6,6 +6,7 @@
 #include "nph_raw.hpp"
 #include "nph_eventalign.hpp"
 #include "nph_scorereads.hpp"
+#include "nph_polya.hpp"
 #include <cmath>
 #include <chrono>
 #include <cstring>
@@ -759,4 +760,51 @@ long long nphh_aligned_segments(int ref_pos, const uint32_t* cigar, int n_cigar,
     return rc ? rc : n;
 }
 
+// ---- N5: polya ------------------------------------------------------------------------------------------------
+// PolyaEstimator over the reads [first_read, first_read + n) of g_reads (names from SquiggleRead::read_name, one contig):
+// add_read / run / tsv.  Returns the TSV's length (written to out if it fits cap) or a negative status.
+long long nphh_polya_tsv(int first_read, int n, const char* contig, const int32_t* positions, const uint16_t* flags,
+                         const uint32_t* suffix_clip, int header, char* out, size_t cap)
+{
+    long long len = -1;
+    int rc = guard([&] {
+        PolyaEstimator est;
+        for (int i = 0; i < n; ++i) {
+            const SquiggleRead& sr = *g_reads[first_read + i];
+            est.add_read(PolyaRecord{sr.read_name, contig, positions[i], flags[i], suffix_clip[i]}, sr);
+        }
+        est.run(Engine::thread_default());
+        const std::string t = est.tsv(header != 0);
+        if (t.size() <= cap) memcpy(out, t.data(), t.size());
+        len = (long long)t.size();
+    });
+    return rc ? rc : len;
+}
+
+// polya_from_raw over raw reads given as nphh_load_from_raw takes them (reads named "read<i>", nucleotide type from
+// nphh_set_rna); returns the TSV's length (written to out if it fits cap) or a negative status
+long long nphh_polya_from_raw(int model, int n, const float* samples, const uint64_t* sample_off, const char* seqs, const uint64_t* seq_off,
+                              double sample_rate, const char* contig, const int32_t* positions, const uint16_t* flags,
+                              const uint32_t* suffix_clip, int header, char* out, size_t cap)
+{
+    long long len = -1;
+    int rc = guard([&] {
+        std::vector<RawRead> raw(n);
+        std::vector<PolyaRecord> recs(n);
+        for (int i = 0; i < n; ++i) {
+            raw[i].read_name = "read" + std::to_string(i);
+            raw[i].read_sequence.assign(seqs + seq_off[i], seqs + seq_off[i + 1]);
+            raw[i].samples.assign(samples + sample_off[i], samples + sample_off[i + 1]);
+            raw[i].sample_rate = sample_rate;
+            raw[i].nucleotide_type = g_raw_is_rna ? SRNT_RNA : SRNT_DNA;
+            recs[i] = PolyaRecord{raw[i].read_name, contig, positions[i], flags[i], suffix_clip[i]};
+        }
+        const std::string t = polya_from_raw(Engine::thread_default(), *g_models[model], raw, recs, header != 0);
+        if (t.size() <= cap) memcpy(out, t.data(), t.size());
+        len = (long long)t.size();
+    });
+    return rc ? rc : len;
+}
+
 } // extern "C"
+

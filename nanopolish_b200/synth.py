@@ -632,3 +632,100 @@ def gen_pileup(ref_len: int, depth: int, read_bases: int, model: PoreModel, seed
         eoff += E; doff += read_bases; poff += pr.shape[0]
     rs = ReadSet(reads, np.concatenate(means), np.concatenate(times), seqs, evk, kfe, k)
     return ref, rs, recs, np.concatenate(prs)
+
+
+# ---- poly(A) tail length (section 8f N5: `nanopolish polya`) ---------------------------------------------------------------
+POLYA_JOB_DT = np.dtype([("sample_off", "<u8"), ("event_off", "<u8"), ("map_off", "<u8"), ("n_samples", "<u4"), ("n_events", "<u4"),
+                         ("n_kmers", "<u4"), ("reserved", "<u4"), ("sample_rate", "<f8"), ("shift", "<f8"), ("scale", "<f8"),
+                         ("var", "<f8")], align=True)
+POLYA_RES_DT = np.dtype([("start", "<u8"), ("leader", "<u8"), ("adapter", "<u8"), ("polya", "<u8"), ("cliffs", "<u8"),
+                         ("read_rate", "<f8"), ("polya_length", "<f8"), ("end_score", "<f4"), ("qc", "<u4")], align=True)
+POLYA_NOREGION, POLYA_ADAPTER, POLYA_FAILED_LOAD = 1, 2, 4
+
+# the reads' families: what each exercises in estimate_polya_for_single_read
+POLYA_FAMILIES = ("pass", "noregion", "adapter", "suffclip", "missing", "zero_median", "failed_load", "tiny")
+
+
+@dataclass
+class PolyaSet:
+    samples: np.ndarray          # f32, every read's trimmed raw samples in acquisition order (3'->5' for direct RNA)
+    durations: np.ndarray        # f32 event durations (seconds), SquiggleRead order
+    map: np.ndarray              # EVENT_RANGE_DT base_to_event_map entries
+    jobs: np.ndarray             # POLYA_JOB_DT
+    names: list
+    suffix_clip: np.ndarray      # u4, length of each record's last CIGAR op
+    family: list
+
+
+def _polya_trace(rng, n_lead, n_adapt, n_polya, n_tx, shift, scale, var, cliff_rate=0.002):
+    """START (Gaussian + uniform), leader, adapter mixture, poly(A) with cliff excursions, then a 5-mer-like transcript;
+    levels in the HMM's unscaled picoamps, mapped through shift + scale * level with var-scaled noise."""
+    n_start = int(rng.integers(150, 1500))
+    s = np.where(rng.random(n_start) < 0.5, rng.normal(70.2737, 3.7743, n_start), rng.uniform(40.0, 250.0, n_start))
+    lead = rng.normal(110.973, 5.237, n_lead)
+    pick = rng.random(n_adapt) < 0.874
+    adapt = np.where(pick, rng.normal(79.347, 8.3702, n_adapt), rng.normal(63.3126, 2.7464, n_adapt))
+    pa = rng.normal(108.883, 3.257, n_polya)
+    cl = rng.random(n_polya) < cliff_rate
+    pa[cl] = rng.uniform(72.0, 95.0, int(cl.sum()))
+    dwell = np.maximum(1, rng.geometric(1.0 / 30.0, n_tx // 20 + 2))
+    lv = np.repeat(rng.uniform(70.0, 125.0, dwell.shape[0]), dwell)[:n_tx]
+    tx = lv + rng.normal(0.0, 2.5, lv.shape[0])
+    lv = np.concatenate([s, lead, adapt, pa, tx])
+    return (shift + scale * lv + (var - 1.0) * rng.normal(0.0, 1.5, lv.shape[0])).astype(np.float32)
+
+
+def gen_polya(n_reads: int, seed: int = 5, families=POLYA_FAMILIES, polya_samples=(2000, 9000), tx_samples=(4000, 20000),
+              sample_rate: float = 3012.0, lengths=None) -> PolyaSet:
+    """Seeded direct-RNA-shaped reads for `polya`, cycling through `families` (POLYA_FAMILIES).  lengths: the trace length of
+    each read instead (cut from, or padded with, transcript)."""
+    samples, durs, maps, names, clips, fam = [], [], [], [], [], []
+    jobs = np.zeros(n_reads, POLYA_JOB_DT)
+    so = eo = mo = 0
+    for r in range(n_reads):
+        rng = np.random.default_rng(seed * 100003 + r)
+        f = families[r % len(families)]
+        shift, scale, var = float(rng.normal(0.0, 3.0)), float(rng.uniform(0.9, 1.1)), float(rng.uniform(0.9, 1.3))
+        n_lead, n_adapt = int(rng.integers(300, 1200)), int(rng.integers(1500, 5000))
+        n_polya, n_tx = int(rng.integers(*polya_samples)), int(rng.integers(*tx_samples))
+        if f == "noregion":
+            n_polya = int(rng.integers(20, 150))
+        elif f == "adapter":
+            n_adapt = int(rng.integers(16000, 24000))
+        elif f == "missing":
+            n_lead = n_adapt = n_polya = 0
+        if f == "tiny":
+            n_tiny = 2 if r < len(families) else int(rng.integers(3, 40))          # n = 2: size_t wrap-around in the defaults
+            x = (shift + scale * rng.uniform(40.0, 210.0, n_tiny)).astype(np.float32)
+        else:
+            x = _polya_trace(rng, n_lead, n_adapt, n_polya, n_tx, shift, scale, var)
+            if f == "missing":
+                x = x[-n_tx:]
+        if lengths is not None and f != "tiny":
+            want = int(lengths[r])
+            x = _polya_trace(rng, n_lead, n_adapt, n_polya, max(16, want), shift, scale, var)[:want]
+        n_kmers = int(rng.integers(300, 2500)) if f != "tiny" else int(rng.integers(1, 8))
+        n_events = 0 if f == "failed_load" else int(n_kmers * rng.uniform(1.2, 2.0)) + 1
+        d = (rng.integers(3, 60, n_events) / sample_rate).astype(np.float32)
+        m = np.zeros(n_kmers, EVENT_RANGE_DT)
+        if n_events:
+            # monotone event ranges per k-mer; some k-mers get none (-1)
+            cuts = np.sort(rng.integers(0, n_events, n_kmers))
+            span = rng.integers(0, 3, n_kmers)
+            m["start"] = cuts
+            m["stop"] = np.minimum(cuts + span, n_events - 1)
+            none = rng.random(n_kmers) < (0.7 if f == "zero_median" else 0.05)
+            m["start"][none] = -1; m["stop"][none] = -1
+        jobs[r] = (so, eo, mo, x.shape[0], n_events, n_kmers, 0, sample_rate, shift, scale, var)
+        samples.append(x); durs.append(d); maps.append(m)
+        names.append(f"{uuid_like(rng)}"); clips.append(int(rng.integers(201, 600)) if f == "suffclip" else int(rng.integers(0, 200)))
+        fam.append(f)
+        so += x.shape[0]; eo += n_events; mo += n_kmers
+    return PolyaSet(np.concatenate(samples), np.concatenate(durs) if eo else np.zeros(0, np.float32), np.concatenate(maps), jobs,
+                    names, np.asarray(clips, np.uint32), fam)
+
+
+def uuid_like(rng) -> str:
+    h = rng.integers(0, 16, 32)
+    s = "".join("0123456789abcdef"[int(v)] for v in h)
+    return f"{s[:8]}-{s[8:12]}-{s[12:16]}-{s[16:20]}-{s[20:]}"
