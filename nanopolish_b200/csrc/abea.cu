@@ -27,8 +27,6 @@
 #include <cmath>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 #ifndef NPH_ABEA_WARPS
@@ -429,6 +427,14 @@ int validate_abea_jobs(nph_ctx* ctx, const nph_abea_job* jobs, size_t n_jobs, si
     return NPH_OK;
 }
 
+// ABEA's band storage in ctx->d_arena: per warp, the k-mer parameters and the trace
+void abea_layout(NphCarve& a, const nph_ctx* ctx, AbeaParams& p)
+{
+    const size_t warps = (size_t)ctx->sm_count * kWarps;
+    p.scratch_params = a.take<float4>((size_t)ctx->abea_kmax * warps);
+    p.scratch_trace = a.take<uint8_t>(ctx->abea_trace_stride * warps);
+}
+
 } // namespace
 
 int nph_launch_abea(nph_ctx* ctx)
@@ -445,11 +451,9 @@ int nph_launch_abea(nph_ctx* ctx)
     p.counter = ctx->d_counters.p + (NPH_NUM_COUNTERS - 1);
     p.pairs = ctx->d_pairs.p;
     p.results = ctx->d_abea_res.p;
-    const int warps = ctx->sm_count * kWarps;
     p.kmax_stride = ctx->abea_kmax;
     p.trace_stride = ctx->abea_trace_stride;
-    p.scratch_params = reinterpret_cast<float4*>(ctx->d_abea_scratch.p);
-    p.scratch_trace = ctx->d_abea_scratch.p + sizeof(float4) * (size_t)p.kmax_stride * warps;
+    NPH_TRY(nph_carve(ctx, ctx->d_arena, [&](NphCarve& a) { abea_layout(a, ctx, p); }));
     p.consts = reinterpret_cast<const AbeaJobConsts*>(ctx->d_abea_consts.p);
     p.lp_skip = log(1e-10);
     p.lp_trim = log(0.01);
@@ -494,7 +498,7 @@ int nph_abea_jobs_load(nph_ctx* ctx, const uint32_t* kmer_ranks, size_t n_ranks_
 
     // per-job transition penalties, evaluated with the host libm in FP64 exactly as raw_loader.cpp:95-108
     std::vector<AbeaJobConsts> consts(n_jobs);
-    std::vector<std::pair<uint64_t, uint32_t>> keyed(n_jobs);
+    std::vector<uint64_t> bands(n_jobs);
     uint32_t kmax = 1;
     uint64_t max_bands = 4;
     const double lp_skip = log(1e-10);
@@ -504,21 +508,17 @@ int nph_abea_jobs_load(nph_ctx* ctx, const uint32_t* kmer_ranks, size_t n_ranks_
         const double p_stay = 1 - (1 / (events_per_kmer + 1));
         consts[j].lp_stay = log(p_stay);
         consts[j].lp_step = log(1.0 - exp(lp_skip) - exp(consts[j].lp_stay));
-        const uint64_t bands = (uint64_t)ctx->h_read_n_events[jobs[j].read] + jobs[j].n_kmers + 2;
-        keyed[j] = {bands, (uint32_t)j};
+        bands[j] = (uint64_t)ctx->h_read_n_events[jobs[j].read] + jobs[j].n_kmers + 2;
         kmax = std::max(kmax, jobs[j].n_kmers);
-        max_bands = std::max(max_bands, bands);
+        max_bands = std::max(max_bands, bands[j]);
     }
-    std::sort(keyed.begin(), keyed.end(), [](const std::pair<uint64_t, uint32_t>& a, const std::pair<uint64_t, uint32_t>& b) {
-        return a.first != b.first ? a.first > b.first : a.second < b.second; });   // longest reads first
-    std::vector<uint32_t> order(n_jobs);
-    for (size_t j = 0; j < n_jobs; ++j) order[j] = keyed[j].second;
+    const std::vector<uint32_t> order = longest_first(bands);   // longest reads first
 
-    const int warps = ctx->sm_count * kWarps;
     ctx->abea_kmax = kmax;
     ctx->abea_trace_stride = 32 * (max_bands + kTraceBlockRows);
-    const size_t scratch = (sizeof(float4) * (size_t)kmax + ctx->abea_trace_stride) * warps;
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, scratch));
+    // ABEA owns the arena (this load sets abea_loaded below); the pointers abea_layout writes into p are not needed here
+    AbeaParams p{};
+    NPH_TRY(nph_reserve(ctx, ctx->d_arena, nph_measure([&](NphCarve& a) { abea_layout(a, ctx, p); })));
     NPH_TRY(nph_reserve(ctx, ctx->d_abea_jobs, n_jobs));
     NPH_TRY(nph_reserve(ctx, ctx->d_abea_ranks, n_ranks_total));
     NPH_TRY(nph_reserve(ctx, ctx->d_abea_order, n_jobs));

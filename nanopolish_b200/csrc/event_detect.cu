@@ -22,8 +22,6 @@
 #include <vector>
 #include <cstdlib>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 constexpr int kThreads = 128;
@@ -648,68 +646,58 @@ __global__ void __launch_bounds__(256) ed_events_kernel(const FastParams p)
 
 } // namespace
 
-static inline size_t ed_al(size_t v) { return (v + 255) / 256 * 256; }
-
-// Scratch the detector needs next to the raw samples (which the caller keeps on the device).
-size_t nph_ed_scratch_bytes(size_t n_samples_total, size_t n_reads, size_t events_total)
+EdScratch nph_ed_layout(NphCarve& a, size_t n_reads, size_t events_total)
 {
-    (void)n_samples_total;                 // nothing per sample any more: the t-statistics never leave the SM
-    const size_t b_n = ed_al(sizeof(uint32_t) * n_reads);
-    return ed_al(sizeof(nph_raw_read) * n_reads) + b_n /*order*/ + ed_al(sizeof(nph_event) * events_total) + 2 * b_n /*n_events, n_peaks*/ + 256 +
-           ed_al(sizeof(uint32_t) * events_total) /*peaks*/ + ed_al(n_reads) /*exact*/;
+    EdScratch s;
+    s.reads = a.take<nph_raw_read>(n_reads);
+    s.order = a.take<uint32_t>(n_reads);
+    s.events = a.take<nph_event>(events_total);
+    s.n_events = a.take<uint32_t>(n_reads);
+    s.ctl = a.take<EdControl>(1);
+    s.peaks = a.take<uint32_t>(events_total);
+    s.n_peaks = a.take<uint32_t>(n_reads);
+    s.exact = a.take<uint8_t>(n_reads);
+    return s;
 }
 
-// Event detection over reads whose samples are already on the device.  Leaves the events (at each read's event_off)
-// and the counts on the device, returns the counts on the host too.  Synchronises the stream (twice: the list of reads
-// that need the sequential fallback, then the counts).
+// Event detection over reads whose samples are already on the device, in the scratch of nph_ed_layout.  Returns the
+// counts on the host too.  Synchronises the stream (twice: the list of reads that need the sequential fallback, then the
+// counts).
 int nph_detect_events_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_total, const nph_raw_read* reads, size_t n_reads,
-                             const nph_event_params* params, uint8_t* scratch, size_t events_total,
-                             nph_event** d_events_out, uint32_t** d_n_events_out, std::vector<uint32_t>& h_n_events, int* launches_out)
+                             const nph_event_params* params, const EdScratch& s, size_t events_total,
+                             std::vector<uint32_t>& h_n_events, int* launches_out)
 {
     if (params->window_length2 > kMaxW2 || params->window_length1 > params->window_length2 || params->window_length1 == 0) return NPH_ERR_UNSUPPORTED;
-    std::vector<std::pair<uint32_t, uint32_t>> keyed(n_reads);
+    std::vector<uint32_t> n_samples(n_reads);
     for (size_t i = 0; i < n_reads; ++i) {
         const nph_raw_read& r = reads[i];
         if (r.n_samples == 0 || r.sample_off + r.n_samples > n_samples_total || r.event_off + r.event_cap > events_total || r.event_cap == 0)
             return NPH_ERR_INVALID;
         if (r.n_samples > 0xFFFFFF00u) return NPH_ERR_UNSUPPORTED;      // position arithmetic is 32-bit with a 2*w2 halo
-        keyed[i] = {r.n_samples, (uint32_t)i};
+        n_samples[i] = r.n_samples;
     }
     // threads of a warp walk reads of similar length: longest first
-    std::sort(keyed.begin(), keyed.end(), [](const std::pair<uint32_t, uint32_t>& a, const std::pair<uint32_t, uint32_t>& b) {
-        return a.first != b.first ? a.first > b.first : a.second < b.second; });
-    std::vector<uint32_t> order(n_reads);
-    for (size_t i = 0; i < n_reads; ++i) order[i] = keyed[i].second;
+    const std::vector<uint32_t> order = longest_first(n_samples);
 
-    const size_t b_reads = ed_al(sizeof(nph_raw_read) * n_reads), b_n = ed_al(sizeof(uint32_t) * n_reads);
-    const size_t b_ev = ed_al(sizeof(nph_event) * events_total), b_pk = ed_al(sizeof(uint32_t) * events_total);
-    uint8_t* base = scratch;
     DetParams p{};
-    nph_raw_read* d_reads = reinterpret_cast<nph_raw_read*>(base); base += b_reads;
-    uint32_t* d_order = reinterpret_cast<uint32_t*>(base); base += b_n;
-    p.events = reinterpret_cast<nph_event*>(base); base += b_ev;
-    p.n_events = reinterpret_cast<uint32_t*>(base); base += b_n;
-    p.overflow = reinterpret_cast<int*>(base); base += 256;
-    uint32_t* d_peaks = reinterpret_cast<uint32_t*>(base); base += b_pk;
-    uint32_t* d_npeaks = reinterpret_cast<uint32_t*>(base); base += b_n;
-    uint8_t* d_exact = reinterpret_cast<uint8_t*>(base);
-    p.raw = d_raw; p.reads = d_reads; p.order = d_order; p.n_reads = (uint32_t)n_reads;
+    p.events = s.events; p.n_events = s.n_events; p.overflow = &s.ctl->overflow;
+    p.raw = d_raw; p.reads = s.reads; p.order = s.order; p.n_reads = (uint32_t)n_reads;
     p.w1 = params->window_length1; p.w2 = params->window_length2;
     p.t1 = params->threshold1; p.t2 = params->threshold2; p.peak_height = params->peak_height;
     p.ring = 2 * p.w2 + 1;
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_reads, reads, sizeof(nph_raw_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_order, order.data(), sizeof(uint32_t) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemsetAsync(p.overflow, 0, 64, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(s.reads, reads, sizeof(nph_raw_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(s.order, order.data(), sizeof(uint32_t) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemsetAsync(s.ctl, 0, nph_align256(sizeof(EdControl)), ctx->stream));     // the slice's whole extent
     // fast path first (fused guard + t-statistics + peaks, then events); reads that fail the exactness guard take the stream kernel
     FastParams f{};
-    f.raw = d_raw; f.reads = d_reads; f.order = d_order; f.n_reads = (uint32_t)n_reads;
-    f.peaks = d_peaks; f.n_peaks = d_npeaks; f.exact = d_exact;
+    f.raw = d_raw; f.reads = s.reads; f.order = s.order; f.n_reads = (uint32_t)n_reads;
+    f.peaks = s.peaks; f.n_peaks = s.n_peaks; f.exact = s.exact;
     f.events = p.events; f.n_events = p.n_events; f.overflow = p.overflow;
-    f.stats = reinterpret_cast<uint32_t*>(p.overflow) + 2;
+    f.stats = s.ctl->stats;
     f.w1 = p.w1; f.w2 = p.w2; f.t1 = p.t1; f.t2 = p.t2; f.peak_height = p.peak_height;
     int launches = 0;
     if (p.w2 > (uint32_t)kFusedMaxW2) {
-        NPH_CUDA(ctx, cudaMemsetAsync(d_exact, 0, n_reads, ctx->stream));   // windows wider than the staged row: every read streams
+        NPH_CUDA(ctx, cudaMemsetAsync(s.exact, 0, n_reads, ctx->stream));   // windows wider than the staged row: every read streams
     } else {
         // one pass over the samples: guard + t-statistics + peaks (ed_fused_kernel)
         TsConsts tc{};
@@ -721,7 +709,7 @@ int nph_detect_events_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_
         // with 1 / 2 / 4), more for small batches (512 reads: 1.46 / 1.02 / 0.86 ms) as long as a segment stays >= 2 warm-ups long
         int wpr = 1;
         const size_t want = (size_t)ctx->sm_count * 20;
-        while (wpr < 4 && n_reads * wpr < want && keyed[0].first / (64u * wpr) >= 2 * f.warm) wpr *= 2;
+        while (wpr < 4 && n_reads * wpr < want && n_samples[order[0]] / (64u * wpr) >= 2 * f.warm) wpr *= 2;
         if (getenv("NPH_EVENTS_WPR")) wpr = atoi(getenv("NPH_EVENTS_WPR"));
         if (wpr >= 4) launch_fused<4>(f, tc, n_reads, ctx->stream);
         else if (wpr == 2) launch_fused<2>(f, tc, n_reads, ctx->stream);
@@ -733,12 +721,12 @@ int nph_detect_events_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_
     NPH_CUDA(ctx, cudaGetLastError());
     // fallback list
     std::vector<uint8_t> exact(n_reads);
-    NPH_CUDA(ctx, cudaMemcpyAsync(exact.data(), d_exact, n_reads, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(exact.data(), s.exact, n_reads, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     std::vector<uint32_t> slow;
     for (size_t t = 0; t < n_reads; ++t) if (!exact[order[t]] || getenv("NPH_EVENTS_FORCE_STREAM")) slow.push_back(order[t]);
     if (!slow.empty()) {
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_order, slow.data(), sizeof(uint32_t) * slow.size(), cudaMemcpyHostToDevice, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(s.order, slow.data(), sizeof(uint32_t) * slow.size(), cudaMemcpyHostToDevice, ctx->stream));
         p.n_reads = (uint32_t)slow.size();
         const size_t smem = sizeof(double) * 2 * p.ring * kThreads;
         NPH_CUDA(ctx, cudaFuncSetAttribute(detect_events_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -756,8 +744,6 @@ int nph_detect_events_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_
         cudaMemcpy(st, f.stats, sizeof(st), cudaMemcpyDeviceToHost);
         fprintf(stderr, "[nph events] reads %zu  repair walks %u  streaming fallback %zu (guard/slice %u)\n", n_reads, st[0], slow.size(), st[1]);
     }
-    *d_events_out = p.events;
-    *d_n_events_out = p.n_events;
     if (launches_out) *launches_out = launches;
     return overflow ? NPH_ERR_UNSUPPORTED : NPH_OK;
 }
@@ -769,20 +755,17 @@ extern "C" int nph_detect_events_batch(nph_ctx* ctx, const float* raw, size_t n_
     if (n_reads == 0) return NPH_OK;
     if (!raw || !reads || !events_out || !n_events_out) return NPH_ERR_INVALID;
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t b_raw = ed_al(sizeof(float) * n_samples_total);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, b_raw + nph_ed_scratch_bytes(n_samples_total, n_reads, events_total)));
-    ctx->abea_loaded = false;     // the arena is shared with the ABEA trace
-    float* d_raw = reinterpret_cast<float*>(ctx->d_abea_scratch.p);
+    float* d_raw = nullptr;
+    EdScratch es;
+    auto layout = [&](NphCarve& a) { d_raw = a.take<float>(n_samples_total); es = nph_ed_layout(a, n_reads, events_total); };
+    NPH_TRY(nph_borrow_arena(ctx, layout));
     NPH_CUDA(ctx, cudaMemcpyAsync(d_raw, raw, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    nph_event* d_events = nullptr;
-    uint32_t* d_n = nullptr;
     std::vector<uint32_t> counts;
     int launches = 0;
-    const int rc = nph_detect_events_device(ctx, d_raw, n_samples_total, reads, n_reads, params, ctx->d_abea_scratch.p + b_raw, events_total,
-                                            &d_events, &d_n, counts, &launches);
+    const int rc = nph_detect_events_device(ctx, d_raw, n_samples_total, reads, n_reads, params, es, events_total, counts, &launches);
     if (rc != NPH_OK && rc != NPH_ERR_UNSUPPORTED) return rc;
-    if (!d_events) return rc;                       // parameters refused before anything ran
+    if (!launches) return rc;                       // parameters refused before anything ran
     ctx->last_launches = launches;
     ctx->timing_valid = true;
     // only the events that exist cross PCIe: a read's room (n_samples / 2 in practice) is ~4.5 x what it fills, and the room of a
@@ -792,10 +775,10 @@ extern "C" int nph_detect_events_batch(nph_ctx* ctx, const float* raw, size_t n_
     if (used * 2 < events_total && n_reads <= 65536) {
         for (size_t i = 0; i < n_reads; ++i)
             if (counts[i])
-                NPH_CUDA(ctx, cudaMemcpyAsync(events_out + reads[i].event_off, d_events + reads[i].event_off, sizeof(nph_event) * counts[i],
+                NPH_CUDA(ctx, cudaMemcpyAsync(events_out + reads[i].event_off, es.events + reads[i].event_off, sizeof(nph_event) * counts[i],
                                               cudaMemcpyDeviceToHost, ctx->stream));
     } else {
-        NPH_CUDA(ctx, cudaMemcpyAsync(events_out, d_events, sizeof(nph_event) * events_total, cudaMemcpyDeviceToHost, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(events_out, es.events, sizeof(nph_event) * events_total, cudaMemcpyDeviceToHost, ctx->stream));
     }
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     std::copy(counts.begin(), counts.end(), n_events_out);

@@ -19,8 +19,6 @@
 #include <algorithm>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 using namespace nph_vit;
@@ -215,8 +213,6 @@ __global__ void __launch_bounds__(kThreads, 1) eventalign_chain_kernel(const Cha
     }
 }
 
-inline size_t al256(size_t v) { return (v + 255) / 256 * 256; }
-
 template <int C>
 void launch_chain(const ChainParams& p, int grid, cudaStream_t stream)
 {
@@ -240,7 +236,7 @@ extern "C" int nph_eventalign_chain(nph_ctx* ctx,
     // validate what the kernel indexes with, and pick the columns per lane: windows span at most kAlignStride + 1
     // reference bases, i.e. kAlignStride + 2 - k k-mers (96 for 6-mers: three columns per lane, every lane busy)
     uint32_t k_min = 255;
-    std::vector<std::pair<uint32_t, uint32_t>> keyed(n_chains);
+    std::vector<uint32_t> n_pairs(n_chains);
     for (size_t i = 0; i < n_chains; ++i) {
         const nph_ea_chain& c = chains[i];
         if (c.read >= ctx->n_reads || c.model_id >= ctx->models.size() || c.k == 0 || c.k != ctx->models[c.model_id].k) return NPH_ERR_INVALID;
@@ -248,12 +244,9 @@ extern "C" int nph_eventalign_chain(nph_ctx* ctx,
         const size_t n_ref_kmers = c.ref_len >= c.k ? (size_t)c.ref_len - c.k + 1 : 0;
         if (c.rank_off + n_ref_kmers > n_ranks_total || c.out_off + c.out_cap > records_total) return NPH_ERR_INVALID;
         k_min = std::min<uint32_t>(k_min, c.k);
-        keyed[i] = {c.n_pairs, (uint32_t)i};
+        n_pairs[i] = c.n_pairs;
     }
-    std::sort(keyed.begin(), keyed.end(), [](const std::pair<uint32_t, uint32_t>& a, const std::pair<uint32_t, uint32_t>& b) {
-        return a.first != b.first ? a.first > b.first : a.second < b.second; });     // longest chains first
-    std::vector<uint32_t> order(n_chains);
-    for (size_t i = 0; i < n_chains; ++i) order[i] = keyed[i].second;
+    const std::vector<uint32_t> order = longest_first(n_pairs);     // longest chains first
     const int cols = (kAlignStride + 2 - (int)k_min) <= 96 ? 3 : 4;
 
     NPH_TRY(nph_upload_read_transitions(ctx, indel_bias));
@@ -268,43 +261,37 @@ extern "C" int nph_eventalign_chain(nph_ctx* ctx,
     const size_t trace_stride = ((size_t)(e_cap + 40) * strip + 63) / 64 * 64;
     const uint32_t states_stride = (uint32_t)(e_cap + strip + 8);
 
-    const size_t b_pairs = sizeof(nph_aligned_pair) * n_pairs_total, b_map = sizeof(int32_t) * n_map_total;
-    const size_t b_ranks = sizeof(uint32_t) * n_ranks_total, b_chains = sizeof(nph_ea_chain) * n_chains;
-    const size_t b_order = sizeof(uint32_t) * n_chains, b_rec = sizeof(nph_ea_record) * records_total;
-    const size_t b_res = sizeof(nph_ea_result) * n_chains;
-    const size_t b_params = sizeof(float4) * strip * warps, b_trace = sizeof(uint16_t) * trace_stride * warps;
-    const size_t b_states = sizeof(nph_align_state) * states_stride * warps;
-    const size_t need = al256(b_pairs) + al256(b_map) + 2 * al256(b_ranks) + al256(b_chains) + al256(b_order) + al256(b_rec) + al256(b_res) +
-                        al256(b_params) + al256(b_trace) + al256(b_states);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, need));        // shares the alignment scratch arena with ABEA / K3
-    ctx->abea_loaded = false;
-    uint8_t* base = ctx->d_abea_scratch.p;
-    auto carve = [&](size_t bytes) { uint8_t* q = base; base += al256(bytes); return q; };
-    nph_aligned_pair* d_pairs = reinterpret_cast<nph_aligned_pair*>(carve(b_pairs));
-    int32_t* d_map = reinterpret_cast<int32_t*>(carve(b_map));
-    uint32_t* d_rf = reinterpret_cast<uint32_t*>(carve(b_ranks));
-    uint32_t* d_rr = reinterpret_cast<uint32_t*>(carve(b_ranks));
-    nph_ea_chain* d_chains = reinterpret_cast<nph_ea_chain*>(carve(b_chains));
-    uint32_t* d_order = reinterpret_cast<uint32_t*>(carve(b_order));
-    nph_ea_record* d_rec = reinterpret_cast<nph_ea_record*>(carve(b_rec));
-    nph_ea_result* d_res = reinterpret_cast<nph_ea_result*>(carve(b_res));
+    struct {
+        nph_aligned_pair* pairs; int32_t* map; uint32_t *rf, *rr; nph_ea_chain* chains; uint32_t* order; nph_ea_record* rec; nph_ea_result* res;
+    } d{};
     ChainParams p{};
-    p.scratch_params = reinterpret_cast<float4*>(carve(b_params));
-    p.scratch_trace = reinterpret_cast<uint16_t*>(carve(b_trace));
-    p.scratch_states = reinterpret_cast<nph_align_state*>(carve(b_states));
+    auto layout = [&](NphCarve& a) {
+        d.pairs = a.take<nph_aligned_pair>(n_pairs_total);
+        d.map = a.take<int32_t>(n_map_total);
+        d.rf = a.take<uint32_t>(n_ranks_total);
+        d.rr = a.take<uint32_t>(n_ranks_total);
+        d.chains = a.take<nph_ea_chain>(n_chains);
+        d.order = a.take<uint32_t>(n_chains);
+        d.rec = a.take<nph_ea_record>(records_total);
+        d.res = a.take<nph_ea_result>(n_chains);
+        p.scratch_params = a.take<float4>(strip * warps);
+        p.scratch_trace = a.take<uint16_t>(trace_stride * warps);
+        p.scratch_states = a.take<nph_align_state>(states_stride * warps);
+    };
+    NPH_TRY(nph_borrow_arena(ctx, layout));
     p.trace_stride = trace_stride; p.states_stride = states_stride; p.e_cap = e_cap;
     p.level = ctx->d_level.p; p.reads = ctx->d_reads.p; p.trans = ctx->d_trans.p; p.models = ctx->d_models.p; p.flank = ctx->d_flank.p;
-    p.pairs = d_pairs; p.map_start = d_map; p.ranks_fwd = d_rf; p.ranks_rc = d_rr; p.chains = d_chains; p.order = d_order;
-    p.n_chains = (uint32_t)n_chains; p.counter = ctx->d_counters.p; p.records = d_rec; p.results = d_res; p.c = ctx->consts;
+    p.pairs = d.pairs; p.map_start = d.map; p.ranks_fwd = d.rf; p.ranks_rc = d.rr; p.chains = d.chains; p.order = d.order;
+    p.n_chains = (uint32_t)n_chains; p.counter = ctx->d_counters.p; p.records = d.rec; p.results = d.res; p.c = ctx->consts;
 
-    if (b_pairs) NPH_CUDA(ctx, cudaMemcpyAsync(d_pairs, pairs, b_pairs, cudaMemcpyHostToDevice, ctx->stream));
-    if (b_map) NPH_CUDA(ctx, cudaMemcpyAsync(d_map, event_map_start, b_map, cudaMemcpyHostToDevice, ctx->stream));
-    if (b_ranks) {
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_rf, ref_ranks_fwd, b_ranks, cudaMemcpyHostToDevice, ctx->stream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_rr, ref_ranks_rc, b_ranks, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_pairs_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.pairs, pairs, sizeof(nph_aligned_pair) * n_pairs_total, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_map_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.map, event_map_start, sizeof(int32_t) * n_map_total, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_ranks_total) {
+        NPH_CUDA(ctx, cudaMemcpyAsync(d.rf, ref_ranks_fwd, sizeof(uint32_t) * n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(d.rr, ref_ranks_rc, sizeof(uint32_t) * n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
     }
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_chains, chains, b_chains, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_order, order.data(), b_order, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.chains, chains, sizeof(nph_ea_chain) * n_chains, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.order, order.data(), sizeof(uint32_t) * n_chains, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, sizeof(unsigned int) * NPH_NUM_COUNTERS, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     if (cols == 3) launch_chain<3>(p, grid, ctx->stream); else launch_chain<4>(p, grid, ctx->stream);
@@ -312,8 +299,8 @@ extern "C" int nph_eventalign_chain(nph_ctx* ctx,
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     ctx->last_launches = 1;
     ctx->timing_valid = 1;
-    if (b_rec) NPH_CUDA(ctx, cudaMemcpyAsync(records_out, d_rec, b_rec, cudaMemcpyDeviceToHost, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(results_out, d_res, b_res, cudaMemcpyDeviceToHost, ctx->stream));
+    if (records_total) NPH_CUDA(ctx, cudaMemcpyAsync(records_out, d.rec, sizeof(nph_ea_record) * records_total, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(results_out, d.res, sizeof(nph_ea_result) * n_chains, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NPH_OK;
 }

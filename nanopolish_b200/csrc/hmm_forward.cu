@@ -31,19 +31,23 @@ __global__ void read_prologue_kernel(const DevRead* __restrict__ reads, const do
 
 } // namespace
 
-static size_t scratch_slice_bytes(const nph_ctx* ctx)
+// One pair of scratch slices per side stream: classes running concurrently on different SMs index their per-warp
+// scratch by (block, warp) and must not share it.
+struct FwdScratch { float4* params; float* edge; };
+
+static void fwd_layout(NphCarve& a, const nph_ctx* ctx, FwdScratch (&s)[nph_ctx::kSideStreams])
 {
-    const int warps = ctx->sm_count * kMaxWarpsPerCta;
-    const size_t per_warp = sizeof(float4) * (size_t)ctx->max_kpad + sizeof(float) * 3 * ((size_t)ctx->max_period + 8);
-    return ((per_warp * warps + 255) / 256) * 256;
+    const size_t warps = (size_t)ctx->sm_count * kMaxWarpsPerCta;
+    for (FwdScratch& x : s) {
+        x.params = a.take<float4>((size_t)ctx->max_kpad * warps);
+        x.edge = a.take<float>(3 * ((size_t)ctx->max_period + 8) * warps);
+    }
 }
 
-// One scratch slice per side stream: classes running concurrently on different SMs index their
-// per-warp scratch by (block, warp) and must not share it.
-size_t nph_hmm_scratch_bytes(const nph_ctx* ctx, int* warps_total_out)
+size_t nph_hmm_scratch_bytes(const nph_ctx* ctx)
 {
-    if (warps_total_out) *warps_total_out = ctx->sm_count * kMaxWarpsPerCta;
-    return scratch_slice_bytes(ctx) * nph_ctx::kSideStreams;
+    FwdScratch s[nph_ctx::kSideStreams];
+    return nph_measure([&](NphCarve& a) { fwd_layout(a, ctx, s); });
 }
 
 int nph_launch_read_prologue(nph_ctx* ctx)
@@ -66,19 +70,19 @@ int nph_launch_hmm_forward(nph_ctx* ctx, float* scores_dev)
     p.models = ctx->d_models.p;
     p.ranks = ctx->d_ranks.p;
     p.jobs = ctx->d_jobs.p;
-    p.logsum_g = ctx->d_logsum;
+    p.logsum_g = ctx->d_logsum.p;
     p.flank = ctx->d_flank.p;
     p.scores = scores_dev ? scores_dev : ctx->d_scores.p;
-    const int warps = ctx->sm_count * kMaxWarpsPerCta;
     p.kpad_stride = ctx->max_kpad;
     p.edge_stride = ctx->max_period + 8;
     p.c = ctx->consts;
     p.lsum_bias = NPH_LOGSUM_ADDR_BIAS;
     p.lsum_scale = 4u;
     p.neg_zero = -0.0f;
-    p.progress = (ctx->levels_inflight && ctx->level_chunk_events) ? ctx->d_progress : nullptr;
+    p.progress = (ctx->levels_inflight && ctx->level_chunk_events) ? ctx->d_progress.p : nullptr;
     p.chunk_events = (uint32_t)ctx->level_chunk_events;
-    const size_t slice = scratch_slice_bytes(ctx);
+    FwdScratch scratch[nph_ctx::kSideStreams];
+    NPH_TRY(nph_carve(ctx, ctx->d_scratch, [&](NphCarve& a) { fwd_layout(a, ctx, scratch); }));
 
     NPH_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, sizeof(unsigned int) * NPH_NUM_COUNTERS, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
@@ -96,9 +100,8 @@ int nph_launch_hmm_forward(nph_ctx* ctx, float* scores_dev)
         const int si = (int)(t % nph_ctx::kSideStreams);
         cudaStream_t st = ctx->side[si];
         if (!used[si]) { NPH_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_fork, 0)); used[si] = true; }
-        uint8_t* base = ctx->d_scratch.p + slice * si;
-        p.scratch_params = reinterpret_cast<float4*>(base);
-        p.scratch_edge = reinterpret_cast<float*>(base + sizeof(float4) * (size_t)ctx->max_kpad * warps);
+        p.scratch_params = scratch[si].params;
+        p.scratch_edge = scratch[si].edge;
         int rc = NPH_ERR_STATE;
         switch (cl.group_width) {
             case 4: rc = launch_width<4, false>(ctx, p, cl, (int)ci, st); break;

@@ -24,8 +24,6 @@
 #include <string>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 constexpr int kWarps = 16;
@@ -157,7 +155,7 @@ extern "C" int nph_hmm_align(nph_ctx* ctx,
     NPH_TRY(nph_hmm_jobs_load(ctx, kmer_ranks, n_ranks_total, jobs, n_jobs, indel_bias));
 
     // class per job (columns per lane) and schedule, longest first
-    std::vector<std::vector<std::pair<uint32_t, uint32_t>>> per(kNumVit);
+    std::vector<std::vector<uint32_t>> steps(kNumVit), jobs_of(kNumVit);
     uint32_t max_kpad = 32, max_period = kMinPeriod;
     uint64_t max_trace = 1;
     for (size_t j = 0; j < n_jobs; ++j) {
@@ -171,7 +169,8 @@ extern "C" int nph_hmm_align(nph_ctx* ctx,
             const double cost = (double)st * (120.0 + 70.0 * kVitCols[i]);
             if (cost < best) { best = cost; bi = i; bsteps = st; }
         }
-        per[bi].push_back({bsteps, (uint32_t)j});
+        steps[bi].push_back(bsteps);
+        jobs_of[bi].push_back((uint32_t)j);
         const uint32_t strip = 32u * kVitCols[bi], n_strips = (K + strip - 1) / strip;
         max_kpad = std::max(max_kpad, n_strips * strip);
         max_period = std::max(max_period, std::max<uint32_t>(E, kMinPeriod));
@@ -182,9 +181,7 @@ extern "C" int nph_hmm_align(nph_ctx* ctx,
     size_t first[kNumVit + 1];
     for (int i = 0; i < kNumVit; ++i) {
         first[i] = order.size();
-        std::sort(per[i].begin(), per[i].end(), [](const std::pair<uint32_t, uint32_t>& a, const std::pair<uint32_t, uint32_t>& b) {
-            return a.first != b.first ? a.first > b.first : a.second < b.second; });
-        for (auto& e : per[i]) order.push_back(e.second);
+        for (uint32_t t : longest_first(steps[i])) order.push_back(jobs_of[i][t]);
     }
     first[kNumVit] = order.size();
 
@@ -202,29 +199,23 @@ extern "C" int nph_hmm_align(nph_ctx* ctx,
     const int max_ctas = (int)std::min<uint64_t>((uint64_t)ctx->sm_count, std::max<uint64_t>(1, kTraceBudget / per_cta));
     const int warps = max_ctas * kWarps;
     const size_t total_states = (size_t)states_off[n_jobs];
-    const size_t b_params = sizeof(float4) * (size_t)max_kpad * warps;
-    const size_t b_edge = sizeof(float) * 3 * ((size_t)max_period + 8) * warps;
-    const size_t b_trace = sizeof(uint16_t) * trace_stride * warps;
-    const size_t b_states = sizeof(nph_align_state) * total_states;
-    const size_t b_off = sizeof(uint64_t) * (n_jobs + 1);
-    const size_t b_n = sizeof(uint32_t) * n_jobs;
-    auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-    const size_t need = al(b_params) + al(b_edge) + al(b_trace) + al(b_states) + al(b_off) + al(b_n) + al(sizeof(uint32_t) * n_jobs);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, need));      // shares the alignment scratch arena with ABEA
-    uint8_t* base = ctx->d_abea_scratch.p;
     VitParams p{};
-    p.scratch_params = reinterpret_cast<float4*>(base); base += al(b_params);
-    p.scratch_edge = reinterpret_cast<float*>(base); base += al(b_edge);
-    p.scratch_trace = reinterpret_cast<uint16_t*>(base); base += al(b_trace);
-    p.states = reinterpret_cast<nph_align_state*>(base); base += al(b_states);
-    uint64_t* d_off = reinterpret_cast<uint64_t*>(base); base += al(b_off);
-    p.n_states = reinterpret_cast<uint32_t*>(base); base += al(b_n);
-    uint32_t* d_order = reinterpret_cast<uint32_t*>(base);
-    p.states_off = d_off;
+    uint64_t* d_off = nullptr;
+    uint32_t* d_order = nullptr;
+    auto layout = [&](NphCarve& a) {
+        p.scratch_params = a.take<float4>((size_t)max_kpad * warps);
+        p.scratch_edge = a.take<float>(3 * ((size_t)max_period + 8) * warps);
+        p.scratch_trace = a.take<uint16_t>(trace_stride * warps);
+        p.states = a.take<nph_align_state>(total_states);
+        p.states_off = d_off = a.take<uint64_t>(n_jobs + 1);
+        p.n_states = a.take<uint32_t>(n_jobs);
+        d_order = a.take<uint32_t>(n_jobs);
+    };
+    NPH_TRY(nph_borrow_arena(ctx, layout));
     p.level = ctx->d_level.p; p.reads = ctx->d_reads.p; p.trans = ctx->d_trans.p; p.models = ctx->d_models.p;
     p.ranks = ctx->d_ranks.p; p.jobs = ctx->d_jobs.p; p.flank = ctx->d_flank.p; p.scores = ctx->d_scores.p;
     p.kpad_stride = max_kpad; p.edge_stride = max_period + 8; p.trace_stride = trace_stride; p.c = ctx->consts;
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_off, states_off, b_off, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d_off, states_off, sizeof(uint64_t) * (n_jobs + 1), cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaMemcpyAsync(d_order, order.data(), sizeof(uint32_t) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, sizeof(unsigned int) * NPH_NUM_COUNTERS, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
@@ -247,10 +238,9 @@ extern "C" int nph_hmm_align(nph_ctx* ctx,
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     ctx->last_launches = launches;
     ctx->timing_valid = true;
-    NPH_CUDA(ctx, cudaMemcpyAsync(states_out, p.states, b_states, cudaMemcpyDeviceToHost, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(n_states_out, p.n_states, b_n, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(states_out, p.states, sizeof(nph_align_state) * total_states, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(n_states_out, p.n_states, sizeof(uint32_t) * n_jobs, cudaMemcpyDeviceToHost, ctx->stream));
     if (scores_out) NPH_CUDA(ctx, cudaMemcpyAsync(scores_out, ctx->d_scores.p, sizeof(float) * n_jobs, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->abea_loaded = false;   // the arena was reused
     return NPH_OK;
 }

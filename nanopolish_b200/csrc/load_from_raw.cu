@@ -16,13 +16,9 @@
 #include <cstdlib>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 constexpr int kConvWarps = 8;
-
-inline size_t al256(size_t v) { return (v + 255) / 256 * 256; }
 
 struct ConvParams {
     const nph_event* events;         // capacity layout: read t at cap_off[t]
@@ -123,23 +119,32 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     std::vector<nph_raw_read> rr(n_jobs);
     size_t cap_total = 0;
     for (size_t j = 0; j < n_jobs; ++j) { rr[j] = nph_raw_read{jobs[j].sample_off, 0, jobs[j].n_samples, 0}; cap_total += jobs[j].n_samples / 2 + 8; }
-    const size_t b_raw = al256(sizeof(float) * n_samples_total);
-    const size_t b_trim = nph_trim_scratch_bytes(rr.data(), n_jobs, 100);
-    const size_t b_ed = nph_ed_scratch_bytes(n_samples_total, n_jobs, cap_total);
-    const size_t b_small = al256(sizeof(uint64_t) * n_jobs) * 2 + al256(sizeof(uint32_t) * n_jobs) + al256(sizeof(double) * n_jobs);
+    // the arena holds the trim's scratch, then (from its start again) the detector's and the conversion's per-read arrays;
+    // it is reserved for the larger of the two, the latter as if every read survived the trim whole
+    TrimScratch ts;
+    EdScratch es;
+    struct { uint64_t *cap_off, *out_off; double* rate; } conv{};
+    auto trim_layout = [&](NphCarve& a) { ts = nph_trim_layout(a, rr.data(), n_jobs, 100); };
+    auto ed_layout = [&](NphCarve& a, size_t n_reads, size_t events_total) {
+        es = nph_ed_layout(a, n_reads, events_total);
+        conv.cap_off = a.take<uint64_t>(n_reads);
+        conv.out_off = a.take<uint64_t>(n_reads);
+        conv.rate = a.take<double>(n_reads);
+    };
     // the samples get a buffer of their own so that they outlive the call (nph_polya_after_load reads them)
     nph_ctx::LoadedRaw& kept = ctx->loaded_raw;
     kept.valid = false;
-    NPH_TRY(nph_reserve(ctx, kept.d_raw, std::max<size_t>(b_raw / sizeof(float), 1)));
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, std::max(b_trim, b_ed + b_small)));
+    NPH_TRY(nph_reserve(ctx, kept.d_raw, std::max<size_t>(nph_align256(sizeof(float) * n_samples_total) / sizeof(float), 1)));
+    const size_t arena_bytes = std::max(nph_measure(trim_layout), nph_measure([&](NphCarve& a) { ed_layout(a, n_jobs, cap_total); }));
+    NPH_TRY(nph_borrow_arena(ctx, [&](NphCarve& a) { a.take<uint8_t>(arena_bytes); }));
+    NPH_TRY(nph_carve(ctx, ctx->d_arena, trim_layout));
     float* d_raw = kept.d_raw.p;
-    uint8_t* arena = ctx->d_abea_scratch.p;
     NPH_CUDA(ctx, cudaMemcpyAsync(d_raw, raw, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     int launches = 0;
     float staged_ms = 0.0f, ms = 0.0f;          // device time of the stages, summed (each stage ends in a sync)
     std::vector<nph_raw_range> range(n_jobs);
-    NPH_TRY(nph_trim_device(ctx, d_raw, n_samples_total, rr.data(), n_jobs, 200, 10, 100, 0.0f, arena, range.data())); ++launches;
+    NPH_TRY(nph_trim_device(ctx, d_raw, n_samples_total, rr.data(), n_jobs, 200, 10, 100, 0.0f, ts, range.data())); ++launches;
     ctx->h_last_trim = range;                   // for nph_last_trim_ranges (SRF_LOAD_RAW_SAMPLES keeps rt.raw[rt.start .. rt.end))
     NPH_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1)); staged_ms += ms;
     const bool verbose = getenv("NPH_TIMING") != nullptr;
@@ -179,12 +184,11 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
         tr[t] = nph_raw_read{jobs[j].sample_off + range[j].start, room, ns, ns / 2 + 8};   // >= 3 samples between boundaries
         room += ns / 2 + 8;
     }
-    nph_event* d_events = nullptr;
-    uint32_t* d_counts = nullptr;
+    NPH_TRY(nph_carve(ctx, ctx->d_arena, [&](NphCarve& a) { ed_layout(a, nl, room); }));
     std::vector<uint32_t> counts;
     int ed_launches = 0;
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    NPH_TRY(nph_detect_events_device(ctx, d_raw, n_samples_total, tr.data(), nl, params, arena, room, &d_events, &d_counts, counts, &ed_launches));
+    NPH_TRY(nph_detect_events_device(ctx, d_raw, n_samples_total, tr.data(), nl, params, es, room, counts, &ed_launches));
     launches += ed_launches;
     NPH_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1)); staged_ms += ms;
     if (verbose) fprintf(stderr, "  events %.2f ms", ms);
@@ -217,41 +221,35 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     NPH_TRY(nph_reserve(ctx, ctx->d_ev_time, n_events_total));
     NPH_TRY(nph_reserve(ctx, ctx->d_level, n_events_total));
     NPH_TRY(nph_reserve(ctx, ctx->d_reads, nl));
-    const size_t b_ev4 = al256(sizeof(float) * n_events_total), b_mom = al256(sizeof(double) * 2 * nl), b_views = al256(sizeof(nph_read) * nl);
-    const size_t b_b2e = al256(sizeof(nph_event_range) * n_ranks_total), b_cal = al256(sizeof(nph_calibration) * nl);
-    NPH_TRY(nph_reserve(ctx, ctx->d_prep, 2 * b_ev4 + b_mom + b_views + b_b2e + b_cal + 256));
-    uint8_t* pb = ctx->d_prep.p;
-    float* d_stdv = reinterpret_cast<float*>(pb); pb += b_ev4;
-    float* d_dur = reinterpret_cast<float*>(pb); pb += b_ev4;
-    double* d_mom = reinterpret_cast<double*>(pb); pb += b_mom;
-    nph_read* d_views = reinterpret_cast<nph_read*>(pb); pb += b_views;
-    nph_event_range* d_b2e = reinterpret_cast<nph_event_range*>(pb); pb += b_b2e;
-    nph_calibration* d_cal = reinterpret_cast<nph_calibration*>(pb); pb += b_cal;
-    int* d_bad = reinterpret_cast<int*>(pb);
+    struct { float *stdv, *dur; double* mom; nph_read* views; nph_event_range* b2e; nph_calibration* cal; int* bad; } d{};
+    auto prep_layout = [&](NphCarve& a) {
+        d.stdv = a.take<float>(n_events_total);
+        d.dur = a.take<float>(n_events_total);
+        d.mom = a.take<double>(2 * nl);
+        d.views = a.take<nph_read>(nl);
+        d.b2e = a.take<nph_event_range>(n_ranks_total);
+        d.cal = a.take<nph_calibration>(nl);
+        d.bad = a.take<int>(1);
+    };
+    NPH_TRY(nph_lay_out(ctx, ctx->d_prep, prep_layout));
     {
-        // small per-read arrays behind the detector's scratch (still alive: the events are read from it)
-        uint8_t* sb = arena + b_ed;
-        uint64_t* d_cap_off = reinterpret_cast<uint64_t*>(sb); sb += al256(sizeof(uint64_t) * n_jobs);
-        uint64_t* d_out_off = reinterpret_cast<uint64_t*>(sb); sb += al256(sizeof(uint64_t) * n_jobs);
-        sb += al256(sizeof(uint32_t) * n_jobs);
-        double* d_rate = reinterpret_cast<double*>(sb);
         std::vector<double> rate(nl);
         for (size_t t = 0; t < nl; ++t) rate[t] = jobs[live[t]].sample_rate;
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_cap_off, cap_off.data(), sizeof(uint64_t) * nl, cudaMemcpyHostToDevice, ctx->stream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_out_off, out_off.data(), sizeof(uint64_t) * nl, cudaMemcpyHostToDevice, ctx->stream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(d_rate, rate.data(), sizeof(double) * nl, cudaMemcpyHostToDevice, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(conv.cap_off, cap_off.data(), sizeof(uint64_t) * nl, cudaMemcpyHostToDevice, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(conv.out_off, out_off.data(), sizeof(uint64_t) * nl, cudaMemcpyHostToDevice, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(conv.rate, rate.data(), sizeof(double) * nl, cudaMemcpyHostToDevice, ctx->stream));
         ConvParams cp{};
-        cp.events = d_events; cp.cap_off = d_cap_off; cp.out_off = d_out_off; cp.n_events = d_counts; cp.sample_rate = d_rate; cp.n_reads = (uint32_t)nl; cp.reverse = params->reverse_events ? 1 : 0;
-        cp.mean = ctx->d_ev_mean.p; cp.stdv = d_stdv; cp.duration = d_dur; cp.level = ctx->d_level.p; cp.start_time = ctx->d_ev_time.p; cp.reads = ctx->d_reads.p;
+        cp.events = es.events; cp.cap_off = conv.cap_off; cp.out_off = conv.out_off; cp.n_events = es.n_events; cp.sample_rate = conv.rate; cp.n_reads = (uint32_t)nl; cp.reverse = params->reverse_events ? 1 : 0;
+        cp.mean = ctx->d_ev_mean.p; cp.stdv = d.stdv; cp.duration = d.dur; cp.level = ctx->d_level.p; cp.start_time = ctx->d_ev_time.p; cp.reads = ctx->d_reads.p;
         NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
         convert_kernel<<<(unsigned)std::min<size_t>((nl + kConvWarps - 1) / kConvWarps, (size_t)ctx->sm_count * 8), kConvWarps * 32, 0, ctx->stream>>>(cp); ++launches;
         NPH_CUDA(ctx, cudaGetLastError());
         NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
         // rate[] etc. must outlive the copies: the stream is synchronised below before they go out of scope
         NPH_CUDA(ctx, cudaMemcpyAsync(ev_mean_out, ctx->d_ev_mean.p, sizeof(float) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(ev_stdv_out, d_stdv, sizeof(float) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(ev_stdv_out, d.stdv, sizeof(float) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
         NPH_CUDA(ctx, cudaMemcpyAsync(ev_start_time_out, ctx->d_ev_time.p, sizeof(double) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(ev_duration_out, d_dur, sizeof(float) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(ev_duration_out, d.dur, sizeof(float) * n_events_total, cudaMemcpyDeviceToHost, ctx->stream));
         NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         NPH_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1)); staged_ms += ms;
         if (verbose) fprintf(stderr, "  convert %.2f ms", ms);
@@ -263,9 +261,9 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     ctx->h_read_n_events.assign(counts.begin(), counts.end());
     ctx->reads_loaded = true;                      // for the staged ABEA calls below; cleared again before returning
     int rc = nph_abea_jobs_load(ctx, kmer_ranks, n_ranks_total, aj.data(), nl, model_id, pairs_total);
-    if (rc == NPH_OK) rc = nph_launch_mom(ctx, d_mom, params->reverse_events != 0);
+    if (rc == NPH_OK) rc = nph_launch_mom(ctx, d.mom, params->reverse_events != 0);
     if (rc == NPH_OK) {
-        apply_mom_kernel<<<(unsigned)((nl + 127) / 128), 128, 0, ctx->stream>>>(d_mom, ctx->d_reads.p, d_views, (uint32_t)nl);
+        apply_mom_kernel<<<(unsigned)((nl + 127) / 128), 128, 0, ctx->stream>>>(d.mom, ctx->d_reads.p, d.views, (uint32_t)nl);
         launches += 2;
         if (cudaGetLastError() != cudaSuccess) rc = NPH_ERR_CUDA;
     }
@@ -275,21 +273,21 @@ extern "C" int nph_load_from_raw_batch(nph_ctx* ctx, const float* raw, size_t n_
     if (rc != NPH_OK) return rc;
 
     // ---- 5. base_to_event_map, events_per_base, recalibration, QC ----
-    NPH_CUDA(ctx, cudaMemsetAsync(d_b2e, 0xff, sizeof(nph_event_range) * n_ranks_total, ctx->stream));
+    NPH_CUDA(ctx, cudaMemsetAsync(d.b2e, 0xff, sizeof(nph_event_range) * n_ranks_total, ctx->stream));
     NphCalArgs ca{};
-    ca.ev_mean = ctx->d_ev_mean.p; ca.reads = d_views; ca.ranks = ctx->d_abea_ranks.p; ca.jobs = ctx->d_abea_jobs.p;
+    ca.ev_mean = ctx->d_ev_mean.p; ca.reads = d.views; ca.ranks = ctx->d_abea_ranks.p; ca.jobs = ctx->d_abea_jobs.p;
     ca.results = ctx->d_abea_res.p; ca.pairs = ctx->d_pairs.p; ca.n_jobs = (uint32_t)nl; ca.model_id = model_id;
-    ca.b2e = d_b2e; ca.out = d_cal; ca.bad_input = d_bad;
+    ca.b2e = d.b2e; ca.out = d.cal; ca.bad_input = d.bad;
     NPH_TRY(nph_launch_recalibrate(ctx, ca)); ++launches;
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     std::vector<nph_calibration> cal(nl);
-    NPH_CUDA(ctx, cudaMemcpyAsync(cal.data(), d_cal, sizeof(nph_calibration) * nl, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(cal.data(), d.cal, sizeof(nph_calibration) * nl, cudaMemcpyDeviceToHost, ctx->stream));
     if (base_to_event_out)
-        NPH_CUDA(ctx, cudaMemcpyAsync(base_to_event_out, d_b2e, sizeof(nph_event_range) * n_ranks_total, cudaMemcpyDeviceToHost, ctx->stream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(base_to_event_out, d.b2e, sizeof(nph_event_range) * n_ranks_total, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     for (size_t t = 0; t < nl; ++t) calibrations_out[live[t]] = cal[t];
     kept.event_off.assign(event_off_out, event_off_out + n_jobs + 1);
-    kept.d_duration = d_dur; kept.d_b2e = d_b2e; kept.d_cal = d_cal;
+    kept.d_duration = d.dur; kept.d_b2e = d.b2e; kept.d_cal = d.cal;
     kept.valid = true;
     NPH_CUDA(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1)); staged_ms += ms;     // ev0 was recorded at the ABEA launch
     if (verbose) fprintf(stderr, "  abea+calibration %.2f ms  (total %.2f ms, %zu of %zu reads aligned)\n", ms, staged_ms, nl, n_jobs);

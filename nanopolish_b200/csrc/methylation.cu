@@ -29,8 +29,6 @@
 #include <string>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 constexpr int kWarps = 8;
@@ -719,21 +717,25 @@ extern "C" int nph_methylation_tsv(nph_ctx* ctx, const char* contig, const char*
     const size_t n = m.n_records, contig_len = std::strlen(contig), names_len = name_off[n];
     for (size_t r = 0; r < n; ++r) if (name_off[r] > name_off[r + 1]) { ctx->last_error = "name_off must ascend"; return NPH_ERR_INVALID; }
     // one staging block: contig | names | name offsets | strand flags
-    auto al = [](size_t v) { return (v + 15) / 16 * 16; };
-    const size_t o_names = al(contig_len + 1), o_noff = o_names + al(names_len + 1), o_rev = o_noff + al(sizeof(uint32_t) * (n + 1));
-    NPH_TRY(nph_reserve(ctx, m.d_tsv_in, o_rev + al(n)));
+    struct { char *contig, *names; uint32_t* noff; uint8_t* rev; } d{};
+    auto layout = [&](NphCarve& a) {
+        d.contig = a.take<char>(contig_len + 1);
+        d.names = a.take<char>(names_len + 1);
+        d.noff = a.take<uint32_t>(n + 1);
+        d.rev = a.take<uint8_t>(n);
+    };
+    NPH_TRY(nph_lay_out(ctx, m.d_tsv_in, layout));
     NPH_TRY(nph_reserve(ctx, m.d_tsv_off, 2 * n + 4));
-    uint8_t* in = m.d_tsv_in.p;
-    NPH_CUDA(ctx, cudaMemcpyAsync(in, contig, contig_len, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(in + o_names, read_names, names_len, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(in + o_noff, name_off, sizeof(uint32_t) * (n + 1), cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(in + o_rev, is_reverse, n, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.contig, contig, contig_len, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.names, read_names, names_len, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.noff, name_off, sizeof(uint32_t) * (n + 1), cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.rev, is_reverse, n, cudaMemcpyHostToDevice, ctx->stream));
     uint64_t* rec_bytes = m.d_tsv_off.p;
     uint64_t* rec_off = rec_bytes + n;                                  // n + 1 entries
     int* d_refused = reinterpret_cast<int*>(rec_off + n + 1);
     NPH_CUDA(ctx, cudaMemsetAsync(d_refused, 0, sizeof(int), ctx->stream));
-    TsvArgs a{m.d_sites.p, m.d_counts.p + 3 * n, m.d_records.p, m.d_ref.p, reinterpret_cast<const char*>(in), (uint32_t)contig_len,
-              reinterpret_cast<const char*>(in + o_names), reinterpret_cast<const uint32_t*>(in + o_noff), in + o_rev, m.params.k, (uint32_t)n,
+    TsvArgs a{m.d_sites.p, m.d_counts.p + 3 * n, m.d_records.p, m.d_ref.p, d.contig, (uint32_t)contig_len,
+              d.names, d.noff, d.rev, m.params.k, (uint32_t)n,
               rec_bytes, rec_off, nullptr, d_refused};
     const int grid = (int)std::min<size_t>((n + kWarps - 1) / kWarps, (size_t)ctx->sm_count * 8);
     meth_tsv_kernel<false><<<grid, kThreads, 0, ctx->stream>>>(a);

@@ -19,40 +19,9 @@ int nph_set_cuda_error(nph_ctx* ctx, cudaError_t e, const char* what)
     return NPH_ERR_CUDA;
 }
 
-template <typename T>
-int nph_reserve(nph_ctx* ctx, DevBuf<T>& b, size_t n)
-{
-    if (n <= b.cap && b.p) return NPH_OK;
-    if (b.p) { NPH_CUDA(ctx, cudaFree(b.p)); b.p = nullptr; b.cap = 0; }
-    size_t want = n + n / 8 + 16;
-    NPH_CUDA(ctx, cudaMalloc((void**)&b.p, want * sizeof(T)));
-    b.cap = want;
-    return NPH_OK;
-}
-template int nph_reserve<float>(nph_ctx*, DevBuf<float>&, size_t);
-template int nph_reserve<double>(nph_ctx*, DevBuf<double>&, size_t);
-template int nph_reserve<uint32_t>(nph_ctx*, DevBuf<uint32_t>&, size_t);
-template int nph_reserve<uint8_t>(nph_ctx*, DevBuf<uint8_t>&, size_t);
-template int nph_reserve<uint16_t>(nph_ctx*, DevBuf<uint16_t>&, size_t);
-template int nph_reserve<DevRead>(nph_ctx*, DevBuf<DevRead>&, size_t);
-template int nph_reserve<DevModelView>(nph_ctx*, DevBuf<DevModelView>&, size_t);
-template int nph_reserve<nph_hmm_job>(nph_ctx*, DevBuf<nph_hmm_job>&, size_t);
-template int nph_reserve<float2>(nph_ctx*, DevBuf<float2>&, size_t);
-template int nph_reserve<nph_abea_job>(nph_ctx*, DevBuf<nph_abea_job>&, size_t);
-template int nph_reserve<nph_aligned_pair>(nph_ctx*, DevBuf<nph_aligned_pair>&, size_t);
-template int nph_reserve<nph_abea_result>(nph_ctx*, DevBuf<nph_abea_result>&, size_t);
-template int nph_reserve<uint64_t>(nph_ctx*, DevBuf<uint64_t>&, size_t);
-template int nph_reserve<nph_meth_record>(nph_ctx*, DevBuf<nph_meth_record>&, size_t);
-template int nph_reserve<nph_meth_site>(nph_ctx*, DevBuf<nph_meth_site>&, size_t);
-
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 extern "C" int nph_destroy(nph_ctx* ctx);
 
 namespace {
-
-template <typename T>
-void free_buf(DevBuf<T>& b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
 
 // clip-penalty table (see np_oracle.c:npo_flank_table for the derivation; ref profile_hmm_r9.inl:200-260)
 int ensure_flank(nph_ctx* ctx, size_t n)
@@ -131,7 +100,7 @@ int create_common(nph_ctx** out, int device, bool own_stream, cudaStream_t strea
         cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_reset, cudaEventDisableTiming) != cudaSuccess ||
         cudaStreamCreateWithFlags(&ctx->cstream, cudaStreamNonBlocking) != cudaSuccess) return fail(NPH_ERR_CUDA);
-    if (cudaMalloc((void**)&ctx->d_progress, sizeof(uint32_t)) != cudaSuccess) return fail(NPH_ERR_NOMEM);
+    if (nph_reserve(ctx, ctx->d_progress, 1) != NPH_OK) return fail(NPH_ERR_NOMEM);
     if (cudaMallocHost((void**)&ctx->h_progress_vals, sizeof(uint32_t) * (nph_ctx::kLevelChunks + 1)) != cudaSuccess) {
         ctx->h_progress_vals = nullptr;
         return fail(NPH_ERR_NOMEM);
@@ -146,8 +115,8 @@ int create_common(nph_ctx** out, int device, bool own_stream, cudaStream_t strea
     std::vector<float> tbl(NPH_TBL_SMEM);
     for (int i = 0; i < NPH_LOGSUM_CUT; ++i) tbl[i] = (float)log(1. + exp((double)-i / 1000.f));
     tbl[NPH_LOGSUM_CUT] = 0.0f;
-    if (cudaMalloc((void**)&ctx->d_logsum, sizeof(float) * NPH_TBL_SMEM) != cudaSuccess) return fail(NPH_ERR_NOMEM);
-    if (cudaMemcpy(ctx->d_logsum, tbl.data(), sizeof(float) * NPH_TBL_SMEM, cudaMemcpyHostToDevice) != cudaSuccess) return fail(NPH_ERR_CUDA);
+    if (nph_reserve(ctx, ctx->d_logsum, NPH_TBL_SMEM) != NPH_OK) return fail(NPH_ERR_NOMEM);
+    if (cudaMemcpy(ctx->d_logsum.p, tbl.data(), sizeof(float) * NPH_TBL_SMEM, cudaMemcpyHostToDevice) != cudaSuccess) return fail(NPH_ERR_CUDA);
     const_transitions(ctx->consts);
     if (nph_reserve(ctx, ctx->d_counters, NPH_NUM_COUNTERS) != NPH_OK) return fail(NPH_ERR_NOMEM);
     if (ensure_flank(ctx, 4096) != NPH_OK) return fail(NPH_ERR_CUDA);
@@ -198,28 +167,15 @@ int nph_destroy(nph_ctx* ctx)
     if (!ctx) return NPH_ERR_INVALID;
     cudaSetDevice(ctx->device);
     if (ctx->stream || !ctx->own_stream) cudaStreamSynchronize(ctx->stream);
-    if (ctx->d_logsum) cudaFree(ctx->d_logsum);
-    free_buf(ctx->d_flank); free_buf(ctx->d_models); free_buf(ctx->d_reads); free_buf(ctx->d_ev_mean);
-    free_buf(ctx->d_ev_time); free_buf(ctx->d_level); free_buf(ctx->d_drift); free_buf(ctx->d_ranks); free_buf(ctx->d_codes); free_buf(ctx->d_rank_base);
-    free_buf(ctx->d_jobs); free_buf(ctx->d_trans); free_buf(ctx->d_order); free_buf(ctx->d_scores);
-    free_buf(ctx->d_counters); free_buf(ctx->d_sched_cls); free_buf(ctx->d_sched_bkt); free_buf(ctx->d_sched_hist); free_buf(ctx->d_scratch); free_buf(ctx->d_abea_jobs); free_buf(ctx->d_abea_ranks);
-    free_buf(ctx->d_pairs); free_buf(ctx->d_abea_res); free_buf(ctx->d_abea_scratch); free_buf(ctx->d_abea_order); free_buf(ctx->d_abea_consts); free_buf(ctx->d_prep);
-    free_buf(ctx->loaded_raw.d_raw); free_buf(ctx->d_polya);
-    free_buf(ctx->meth.d_ref); free_buf(ctx->meth.d_pairs); free_buf(ctx->meth.d_records); free_buf(ctx->meth.d_prov_off); free_buf(ctx->meth.d_prov);
-    free_buf(ctx->meth.d_counts); free_buf(ctx->meth.d_sites); free_buf(ctx->meth.d_tsv_in); free_buf(ctx->meth.d_tsv_off); free_buf(ctx->meth.d_tsv); free_buf(ctx->meth.d_deltas); free_buf(ctx->meth.d_dense);
-    free_buf(ctx->screen.d_ref); free_buf(ctx->screen.d_deltas); free_buf(ctx->screen.d_dense); free_buf(ctx->screen.d_records);
-    free_buf(ctx->screen.d_pos_off); free_buf(ctx->screen.d_pos_reads); free_buf(ctx->screen.d_state); free_buf(ctx->screen.d_job_off);
-    for (auto& m : ctx->models) { cudaFree(m.mean); cudaFree(m.stdv); cudaFree(m.log_stdv); }
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
     if (ctx->ev_reset) cudaEventDestroy(ctx->ev_reset);
     if (ctx->cstream) { cudaStreamSynchronize(ctx->cstream); cudaStreamDestroy(ctx->cstream); }
-    if (ctx->d_progress) cudaFree(ctx->d_progress);
     if (ctx->h_progress_vals) cudaFreeHost(ctx->h_progress_vals);
     for (int i = 0; i < nph_ctx::kSideStreams; ++i) { if (ctx->ev_join[i]) cudaEventDestroy(ctx->ev_join[i]); if (ctx->side[i]) cudaStreamDestroy(ctx->side[i]); }
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;                      // the device buffers free themselves
     return NPH_OK;
 }
 
@@ -243,17 +199,17 @@ int nph_model_upload(nph_ctx* ctx, const double* level_mean, const double* level
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
     DevModel m;
     const size_t bytes = sizeof(double) * n_states;
-    NPH_CUDA(ctx, cudaMalloc((void**)&m.mean, bytes));
-    NPH_CUDA(ctx, cudaMalloc((void**)&m.stdv, bytes));
-    NPH_CUDA(ctx, cudaMalloc((void**)&m.log_stdv, bytes));
-    NPH_CUDA(ctx, cudaMemcpyAsync(m.mean, level_mean, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(m.stdv, level_stdv, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(m.log_stdv, level_log_stdv, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_TRY(nph_reserve(ctx, m.mean, n_states));
+    NPH_TRY(nph_reserve(ctx, m.stdv, n_states));
+    NPH_TRY(nph_reserve(ctx, m.log_stdv, n_states));
+    NPH_CUDA(ctx, cudaMemcpyAsync(m.mean.p, level_mean, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(m.stdv.p, level_stdv, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(m.log_stdv.p, level_log_stdv, bytes, cudaMemcpyHostToDevice, ctx->stream));
     m.n_states = n_states; m.k = k; m.alphabet_size = alphabet_size;
-    ctx->models.push_back(m);
+    ctx->models.push_back(std::move(m));
     std::vector<DevModelView> views(ctx->models.size());
     for (size_t i = 0; i < views.size(); ++i)
-        views[i] = DevModelView{ctx->models[i].mean, ctx->models[i].stdv, ctx->models[i].log_stdv, ctx->models[i].n_states,
+        views[i] = DevModelView{ctx->models[i].mean.p, ctx->models[i].stdv.p, ctx->models[i].log_stdv.p, ctx->models[i].n_states,
                                 (uint16_t)ctx->models[i].k, (uint16_t)ctx->models[i].alphabet_size};
     NPH_TRY(nph_reserve(ctx, ctx->d_models, views.size()));
     NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_models.p, views.data(), sizeof(DevModelView) * views.size(), cudaMemcpyHostToDevice, ctx->stream));
@@ -301,7 +257,7 @@ int nph_reads_load_impl(nph_ctx* ctx, const nph_read* reads, size_t n_reads,
         size_t chunk = (n_events_total + nph_ctx::kLevelChunks - 1) / nph_ctx::kLevelChunks;
         chunk = (chunk + 31) / 32 * 32;                       // 128-byte lines never straddle two chunks
         ctx->level_chunk_events = chunk;
-        NPH_CUDA(ctx, cudaMemsetAsync(ctx->d_progress, 0, sizeof(uint32_t), ctx->cstream));
+        NPH_CUDA(ctx, cudaMemsetAsync(ctx->d_progress.p, 0, sizeof(uint32_t), ctx->cstream));
         NPH_CUDA(ctx, cudaEventRecord(ctx->ev_reset, ctx->cstream));
         NPH_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_reset, 0));
         ctx->levels_inflight = true;
@@ -332,7 +288,7 @@ int nph_upload_level_chunks(nph_ctx* ctx, const float* ev_mean)
     for (size_t off = 0; off < total; off += chunk, ++c) {
         const size_t n = std::min(chunk, total - off);
         NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_level.p + off, ev_mean + off, sizeof(float) * n, cudaMemcpyHostToDevice, ctx->cstream));
-        NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_progress, ctx->h_progress_vals + c, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->cstream));
+        NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_progress.p, ctx->h_progress_vals + c, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->cstream));
     }
     return NPH_OK;
 }
@@ -363,22 +319,15 @@ static int jobs_upload_async(nph_ctx* ctx, const uint32_t* kmer_ranks, const uin
     ctx->codes_mode = kmer_ranks == nullptr;
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
 
-    // per-read transition pair (2 logf with the host libm, see read_transitions)
-    std::vector<float2>& trans = ctx->h_stage_trans;
-    trans.resize(ctx->n_reads);
-    for (size_t i = 0; i < ctx->n_reads; ++i) trans[i] = read_transitions(ctx->h_events_per_base[i], indel_bias);
-
     if (ctx->codes_mode) NPH_TRY(nph_reserve(ctx, ctx->d_codes, n_ranks_total + 16));
     else NPH_TRY(nph_reserve(ctx, ctx->d_ranks, n_ranks_total));
     NPH_TRY(nph_reserve(ctx, ctx->d_jobs, n_jobs));
     NPH_TRY(nph_reserve(ctx, ctx->d_order, n_jobs));
-    NPH_TRY(nph_reserve(ctx, ctx->d_trans, ctx->n_reads));
     NPH_TRY(nph_reserve(ctx, ctx->d_scores, n_jobs));
     NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_jobs.p, jobs, sizeof(nph_hmm_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
     if (ctx->codes_mode) NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_codes.p, seq_codes, n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
     else NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_ranks.p, kmer_ranks, sizeof(uint32_t) * n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(ctx->d_trans.p, trans.data(), sizeof(float2) * ctx->n_reads, cudaMemcpyHostToDevice, ctx->stream));
-    return NPH_OK;
+    return nph_upload_read_transitions(ctx, indel_bias);
 }
 
 int nph_jobs_schedule(nph_ctx* ctx, size_t n_jobs, size_t n_ranks_total)
@@ -387,7 +336,7 @@ int nph_jobs_schedule(nph_ctx* ctx, size_t n_jobs, size_t n_ranks_total)
     uint32_t max_E = 1;
     NPH_TRY(nph_schedule_hmm_jobs(ctx, n_jobs, n_ranks_total, &max_E));
     NPH_TRY(ensure_flank(ctx, (size_t)max_E + 2));
-    NPH_TRY(nph_reserve(ctx, ctx->d_scratch, nph_hmm_scratch_bytes(ctx, nullptr)));
+    NPH_TRY(nph_reserve(ctx, ctx->d_scratch, nph_hmm_scratch_bytes(ctx)));
     ctx->n_jobs = n_jobs;
     ctx->n_ranks = n_ranks_total;
     ctx->jobs_loaded = true;

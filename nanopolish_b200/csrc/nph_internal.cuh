@@ -28,20 +28,26 @@ struct HmmConsts {
     float log_inv_sqrt_2pi;
 };
 
-struct DevModel {
-    double* mean = nullptr;
-    double* stdv = nullptr;
-    double* log_stdv = nullptr;
-    uint32_t n_states = 0, k = 0, alphabet_size = 0;
-};
 
 // Device-side view of the models for kernels (array of pointers)
 struct DevModelView { const double* mean; const double* stdv; const double* log_stdv; uint32_t n_states; uint16_t k; uint16_t alphabet_size; };
 
+// A device allocation owned by its holder: freed on destruction, moved but never copied.  Grown by nph_reserve.
 template <typename T>
 struct DevBuf {
     T* p = nullptr;
     size_t cap = 0;   // elements
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~DevBuf() { if (p) cudaFree(p); }
+};
+
+struct DevModel {
+    DevBuf<double> mean, stdv, log_stdv;
+    uint32_t n_states = 0, k = 0, alphabet_size = 0;
 };
 
 struct nph_ctx {
@@ -52,7 +58,7 @@ struct nph_ctx {
     std::string last_error;
 
     // constant tables
-    float* d_logsum = nullptr;       // NPH_TBL_SMEM floats
+    DevBuf<float> d_logsum;          // NPH_TBL_SMEM floats
     DevBuf<float> d_flank;           // clip-penalty table, grown on demand
     std::vector<float> h_flank;
     HmmConsts consts;
@@ -102,7 +108,9 @@ struct nph_ctx {
     DevBuf<uint32_t> d_abea_ranks;
     DevBuf<nph_aligned_pair> d_pairs;
     DevBuf<nph_abea_result> d_abea_res;
-    DevBuf<uint8_t> d_abea_scratch;
+    // ABEA's band storage while an ABEA batch is resident; between batches, the scratch of trim, event detection,
+    // recalibration, Viterbi, eventalign chains and load_from_raw, which take it through nph_borrow_arena
+    DevBuf<uint8_t> d_arena;
     DevBuf<uint32_t> d_abea_order;
     DevBuf<double> d_abea_consts;    // per job (lp_stay, lp_step); also the MoM output buffer
     DevBuf<uint8_t> d_prep;          // load_from_raw: event SoA staging, MoM output, calibration buffers
@@ -165,7 +173,7 @@ struct nph_ctx {
     static const int kLevelChunks = 8;
     cudaStream_t cstream = nullptr;
     cudaEvent_t ev_reset = nullptr;
-    uint32_t* d_progress = nullptr;          // number of level chunks that have landed
+    DevBuf<uint32_t> d_progress;             // number of level chunks that have landed
     uint32_t* h_progress_vals = nullptr;     // pinned {1, 2, ...}: sources of the progress writes
     size_t level_chunk_events = 0;           // 0 = levels fully resident, kernels do not poll
     bool levels_inflight = false;
@@ -194,13 +202,88 @@ struct nph_ctx {
 int nph_set_cuda_error(nph_ctx* ctx, cudaError_t e, const char* what);
 #define NPH_CUDA(ctx, call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return nph_set_cuda_error((ctx), e__, #call); } while (0)
 
+#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
+
 template <typename T>
-int nph_reserve(nph_ctx* ctx, DevBuf<T>& b, size_t n);
+int nph_reserve(nph_ctx* ctx, DevBuf<T>& b, size_t n)
+{
+    if (n <= b.cap && b.p) return NPH_OK;
+    if (b.p) { NPH_CUDA(ctx, cudaFree(b.p)); b.p = nullptr; b.cap = 0; }
+    size_t want = n + n / 8 + 16;
+    NPH_CUDA(ctx, cudaMalloc((void**)&b.p, want * sizeof(T)));
+    b.cap = want;
+    return NPH_OK;
+}
+
+inline size_t nph_align256(size_t bytes) { return (bytes + 255) / 256 * 256; }
+
+// The typed slices of one byte arena, in the order they are taken, each starting on a 256-byte boundary.  A layout is
+// written once, as code that takes its slices from an NphCarve, and run twice: nph_measure runs it without an arena to
+// count the bytes to reserve, nph_carve runs it over the reserved arena to hand out the pointers.
+struct NphCarve {
+    uint8_t* base = nullptr;     // null: measure only (every slice is nullptr)
+    size_t cap = 0, used = 0;
+    template <typename T>
+    T* take(size_t n)
+    {
+        const size_t at = used;
+        used += nph_align256(sizeof(T) * n);
+        return base && used <= cap ? reinterpret_cast<T*>(base + at) : nullptr;
+    }
+};
+
+template <typename F>
+size_t nph_measure(F&& layout)
+{
+    NphCarve c;
+    layout(c);
+    return c.used;
+}
+
+// A layout that does not fit its arena is refused: no slice of it may be used.
+template <typename F>
+int nph_carve(nph_ctx* ctx, const DevBuf<uint8_t>& arena, F&& layout)
+{
+    NphCarve c{arena.p, arena.cap};
+    layout(c);
+    if (c.used <= c.cap) return NPH_OK;
+    ctx->last_error = "internal: a scratch layout of " + std::to_string(c.used) + " bytes exceeds its " + std::to_string(c.cap) + "-byte arena";
+    return NPH_ERR_STATE;
+}
+
+// Grows the arena to what the layout takes, then carves it.
+template <typename F>
+int nph_lay_out(nph_ctx* ctx, DevBuf<uint8_t>& arena, F&& layout)
+{
+    NPH_TRY(nph_reserve(ctx, arena, nph_measure(layout)));
+    return nph_carve(ctx, arena, layout);
+}
+
+// Lays a call's scratch out in ctx->d_arena: the resident ABEA batch, whose band storage the arena holds, is gone.
+template <typename F>
+int nph_borrow_arena(nph_ctx* ctx, F&& layout)
+{
+    ctx->abea_loaded = false;
+    return nph_lay_out(ctx, ctx->d_arena, layout);
+}
+
+// Indices of keys, largest key first, equal keys in ascending index order.
+template <typename K>
+std::vector<uint32_t> longest_first(const std::vector<K>& keys)
+{
+    std::vector<std::pair<K, uint32_t>> keyed(keys.size());
+    for (size_t i = 0; i < keys.size(); ++i) keyed[i] = {keys[i], (uint32_t)i};
+    std::sort(keyed.begin(), keyed.end(), [](const std::pair<K, uint32_t>& a, const std::pair<K, uint32_t>& b) {
+        return a.first != b.first ? a.first > b.first : a.second < b.second; });
+    std::vector<uint32_t> order(keys.size());
+    for (size_t i = 0; i < keys.size(); ++i) order[i] = keyed[i].second;
+    return order;
+}
 
 // kernels (defined in hmm_forward.cu / abea.cu)
 int nph_launch_read_prologue(nph_ctx* ctx);
 int nph_launch_hmm_forward(nph_ctx* ctx, float* scores_dev);
-size_t nph_hmm_scratch_bytes(const nph_ctx* ctx, int* warps_total_out);
+size_t nph_hmm_scratch_bytes(const nph_ctx* ctx);
 int nph_launch_abea(nph_ctx* ctx);
 int nph_schedule_hmm_jobs(nph_ctx* ctx, size_t n_jobs, size_t n_ranks_total, uint32_t* max_E_out);
 // per-read (lp_mm_self, lp_mm_next) of the resident reads into ctx->d_trans (host libm, like calculate_transitions)
@@ -221,13 +304,20 @@ void nph_finish_level_upload(nph_ctx* ctx);
 
 // ---- device-level pieces of the raw-read prologue (event_detect.cu, squiggle_prep.cu, abea.cu), chained by
 // load_from_raw.cu without leaving the device.  Inputs named d_* are device pointers; everything runs on ctx->stream.
-size_t nph_ed_scratch_bytes(size_t n_samples_total, size_t n_reads, size_t events_total);
+struct EdControl { int overflow; uint32_t stats[2]; };   // stats: repair walks, reads that fail the exactness guard
+struct EdScratch {
+    nph_raw_read* reads; uint32_t* order; nph_event* events; uint32_t* n_events; EdControl* ctl; uint32_t* peaks; uint32_t* n_peaks; uint8_t* exact;
+};
+EdScratch nph_ed_layout(NphCarve& a, size_t n_reads, size_t events_total);
+// leaves the events (at each read's event_off) in s.events and the counts in s.n_events; *launches_out stays 0 if the
+// parameters were refused before anything ran
 int nph_detect_events_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_total, const nph_raw_read* reads, size_t n_reads,
-                             const nph_event_params* params, uint8_t* scratch, size_t events_total,
-                             nph_event** d_events_out, uint32_t** d_n_events_out, std::vector<uint32_t>& h_n_events, int* launches_out);
-size_t nph_trim_scratch_bytes(const nph_raw_read* reads, size_t n_reads, int32_t varseg_chunk);
+                             const nph_event_params* params, const EdScratch& s, size_t events_total,
+                             std::vector<uint32_t>& h_n_events, int* launches_out);
+struct TrimScratch { nph_raw_read* reads; uint64_t* mad_off; float* mad; nph_raw_range* out; };
+TrimScratch nph_trim_layout(NphCarve& a, const nph_raw_read* reads, size_t n_reads, int32_t varseg_chunk);
 int nph_trim_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_total, const nph_raw_read* reads, size_t n_reads,
-                    int32_t trim_start, int32_t trim_end, int32_t varseg_chunk, float varseg_thresh, uint8_t* scratch,
+                    int32_t trim_start, int32_t trim_end, int32_t varseg_chunk, float varseg_thresh, const TrimScratch& s,
                     nph_raw_range* ranges_out /* host */);
 struct NphCalArgs {
     const float* ev_mean;

@@ -18,8 +18,6 @@
 #include <cmath>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 using namespace nph_polya_math;
@@ -342,12 +340,10 @@ __global__ void after_load_jobs_kernel(const AfterLoadArgs a)
     a.jobs_out[j] = pj;
 }
 
-inline size_t al256(size_t v) { return (v + 255) / 256 * 256; }
-
 // Per-warp scratch: backpointers (1 B per sample) and per-k-mer durations (8 B per map entry) of the read a warp holds,
 // sized from the batch's longest read.  The grid is the resident warps (at most one per job), fewer if that scratch would
 // exceed the larger of the batch's own footprint and 1 GiB.
-struct ScratchPlan { unsigned blocks = 1; uint64_t bp_stride = 256, kd_stride = 32; size_t bytes = 0; };
+struct ScratchPlan { unsigned blocks = 1; uint64_t bp_stride = 256, kd_stride = 32; };
 
 int plan_scratch(nph_ctx* ctx, const std::vector<nph_polya_job>& jobs, ScratchPlan* plan)
 {
@@ -360,48 +356,50 @@ int plan_scratch(nph_ctx* ctx, const std::vector<nph_polya_job>& jobs, ScratchPl
     int per_sm = 0;
     NPH_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, polya_kernel, kWarps * 32, 0));
     ScratchPlan p;
-    p.bp_stride = al256(max_n);
-    p.kd_stride = al256(8 * max_k) / 8;
+    p.bp_stride = nph_align256(max_n);
+    p.kd_stride = nph_align256(8 * max_k) / 8;
     const uint64_t per_block = kWarps * (p.bp_stride + 8 * p.kd_stride);
     const uint64_t budget = std::max<uint64_t>(sum, 1ull << 30);
     size_t blocks = std::min<size_t>((jobs.size() + kWarps - 1) / kWarps, (size_t)ctx->sm_count * std::max(per_sm, 1));
     blocks = std::max<size_t>(1, std::min<size_t>(blocks, budget / per_block));
     p.blocks = (unsigned)blocks;
-    p.bytes = blocks * per_block;
     *plan = p;
     return NPH_OK;
 }
 
-size_t run_scratch_bytes(size_t n_jobs, const ScratchPlan& plan)
+struct PolyaControl { unsigned int next; int bad; };      // work counter, 1 + index of an invalid job
+
+// run_polya's slices, behind the inputs of its caller
+struct RunScratch { uint32_t* order; nph_polya_result* results; PolyaControl* ctl; double* kmer_dur; uint8_t* bptr; };
+
+RunScratch run_layout(NphCarve& a, size_t n_jobs, const ScratchPlan& plan)
 {
-    return al256(sizeof(uint32_t) * n_jobs) + al256(sizeof(nph_polya_result) * n_jobs) + 256 + plan.bytes;
+    RunScratch s;
+    s.order = a.take<uint32_t>(n_jobs);
+    s.results = a.take<nph_polya_result>(n_jobs);
+    s.ctl = a.take<PolyaControl>(1);
+    s.kmer_dur = a.take<double>((size_t)plan.blocks * kWarps * plan.kd_stride);
+    s.bptr = a.take<uint8_t>((size_t)plan.blocks * kWarps * plan.bp_stride);
+    return s;
 }
 
 // validate, schedule and run the jobs already at d_jobs; samples / durations / map are device pointers
 int run_polya(nph_ctx* ctx, const float* d_samples, size_t n_samples_total, const float* d_dur, size_t n_events_total,
               const nph_event_range* d_map, size_t n_map_total, nph_polya_job* d_jobs, const std::vector<nph_polya_job>& jobs,
-              const ScratchPlan& plan, uint8_t* arena, nph_polya_result* results_out)
+              const ScratchPlan& plan, const RunScratch& s, nph_polya_result* results_out)
 {
     const size_t n_jobs = jobs.size();
-    uint8_t* pb = arena;
-    uint32_t* d_order = reinterpret_cast<uint32_t*>(pb); pb += al256(sizeof(uint32_t) * n_jobs);
-    nph_polya_result* d_res = reinterpret_cast<nph_polya_result*>(pb); pb += al256(sizeof(nph_polya_result) * n_jobs);
-    unsigned int* d_ctl = reinterpret_cast<unsigned int*>(pb); pb += 256;
-    double* d_kmer = reinterpret_cast<double*>(pb); pb += (size_t)plan.blocks * kWarps * plan.kd_stride * 8;
-    uint8_t* d_bp = pb;
-
-    std::vector<uint32_t> order(n_jobs);
-    for (size_t i = 0; i < n_jobs; ++i) order[i] = (uint32_t)i;
-    std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) {
-        return (jobs[x].n_events ? jobs[x].n_samples : 0u) > (jobs[y].n_events ? jobs[y].n_samples : 0u); });
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_order, order.data(), sizeof(uint32_t) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemsetAsync(d_ctl, 0, 256, ctx->stream));
+    std::vector<uint32_t> length(n_jobs);
+    for (size_t i = 0; i < n_jobs; ++i) length[i] = jobs[i].n_events ? jobs[i].n_samples : 0u;
+    const std::vector<uint32_t> order = longest_first(length);
+    NPH_CUDA(ctx, cudaMemcpyAsync(s.order, order.data(), sizeof(uint32_t) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemsetAsync(s.ctl, 0, nph_align256(sizeof(PolyaControl)), ctx->stream));     // the slice's whole extent
 
     PolyaArgs pa{};
-    pa.samples = d_samples; pa.durations = d_dur; pa.map = d_map; pa.jobs = d_jobs; pa.order = d_order; pa.n_jobs = (uint32_t)n_jobs;
+    pa.samples = d_samples; pa.durations = d_dur; pa.map = d_map; pa.jobs = d_jobs; pa.order = s.order; pa.n_jobs = (uint32_t)n_jobs;
     pa.n_samples_total = n_samples_total; pa.n_events_total = n_events_total; pa.n_map_total = n_map_total;
-    pa.bptr = d_bp; pa.kmer_dur = d_kmer; pa.bp_stride = plan.bp_stride; pa.kd_stride = plan.kd_stride;
-    pa.results = d_res; pa.next = d_ctl; pa.bad = reinterpret_cast<int*>(d_ctl + 1);
+    pa.bptr = s.bptr; pa.kmer_dur = s.kmer_dur; pa.bp_stride = plan.bp_stride; pa.kd_stride = plan.kd_stride;
+    pa.results = s.results; pa.next = &s.ctl->next; pa.bad = &s.ctl->bad;
     const unsigned vblocks = (unsigned)std::min<size_t>((n_jobs + kWarps - 1) / kWarps, (size_t)ctx->sm_count * 8);
     polya_validate_kernel<<<vblocks, kWarps * 32, 0, ctx->stream>>>(pa);
     NPH_CUDA(ctx, cudaGetLastError());
@@ -416,7 +414,7 @@ int run_polya(nph_ctx* ctx, const float* d_samples, size_t n_samples_total, cons
     polya_kernel<<<plan.blocks, kWarps * 32, 0, ctx->stream>>>(pa);
     NPH_CUDA(ctx, cudaGetLastError());
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(results_out, d_res, sizeof(nph_polya_result) * n_jobs, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(results_out, s.results, sizeof(nph_polya_result) * n_jobs, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->last_launches = 2;
     ctx->timing_valid = 1;
@@ -437,19 +435,21 @@ extern "C" int nph_polya_batch(nph_ctx* ctx, const float* samples, size_t n_samp
     std::vector<nph_polya_job> hj(jobs, jobs + n_jobs);
     ScratchPlan plan;
     NPH_TRY(plan_scratch(ctx, hj, &plan));
-    const size_t b_s = al256(sizeof(float) * std::max<size_t>(n_samples_total, 1)), b_d = al256(sizeof(float) * std::max<size_t>(n_events_total, 1));
-    const size_t b_m = al256(sizeof(nph_event_range) * std::max<size_t>(n_map_total, 1)), b_j = al256(sizeof(nph_polya_job) * n_jobs);
-    NPH_TRY(nph_reserve(ctx, ctx->d_polya, b_s + b_d + b_m + b_j + run_scratch_bytes(n_jobs, plan)));
-    uint8_t* pb = ctx->d_polya.p;
-    float* d_s = reinterpret_cast<float*>(pb); pb += b_s;
-    float* d_d = reinterpret_cast<float*>(pb); pb += b_d;
-    nph_event_range* d_m = reinterpret_cast<nph_event_range*>(pb); pb += b_m;
-    nph_polya_job* d_j = reinterpret_cast<nph_polya_job*>(pb); pb += b_j;
-    if (n_samples_total) NPH_CUDA(ctx, cudaMemcpyAsync(d_s, samples, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
-    if (n_events_total) NPH_CUDA(ctx, cudaMemcpyAsync(d_d, durations, sizeof(float) * n_events_total, cudaMemcpyHostToDevice, ctx->stream));
-    if (n_map_total) NPH_CUDA(ctx, cudaMemcpyAsync(d_m, map, sizeof(nph_event_range) * n_map_total, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_j, jobs, sizeof(nph_polya_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    return run_polya(ctx, d_s, n_samples_total, d_d, n_events_total, d_m, n_map_total, d_j, hj, plan, pb, results_out);
+    struct { float *samples, *durations; nph_event_range* map; nph_polya_job* jobs; } d{};
+    RunScratch rs;
+    auto layout = [&](NphCarve& a) {
+        d.samples = a.take<float>(std::max<size_t>(n_samples_total, 1));
+        d.durations = a.take<float>(std::max<size_t>(n_events_total, 1));
+        d.map = a.take<nph_event_range>(std::max<size_t>(n_map_total, 1));
+        d.jobs = a.take<nph_polya_job>(n_jobs);
+        rs = run_layout(a, n_jobs, plan);
+    };
+    NPH_TRY(nph_lay_out(ctx, ctx->d_polya, layout));
+    if (n_samples_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.samples, samples, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_events_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.durations, durations, sizeof(float) * n_events_total, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_map_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.map, map, sizeof(nph_event_range) * n_map_total, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.jobs, jobs, sizeof(nph_polya_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    return run_polya(ctx, d.samples, n_samples_total, d.durations, n_events_total, d.map, n_map_total, d.jobs, hj, plan, rs, results_out);
 }
 
 extern "C" int nph_polya_after_load(nph_ctx* ctx, nph_polya_result* results_out, size_t n_jobs)
@@ -459,8 +459,6 @@ extern "C" int nph_polya_after_load(nph_ctx* ctx, nph_polya_result* results_out,
     if (!k.valid || n_jobs != k.jobs.size()) return NPH_ERR_STATE;
     if (n_jobs == 0) return NPH_OK;
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t b_rj = al256(sizeof(nph_raw_job) * n_jobs), b_tr = al256(sizeof(nph_raw_range) * n_jobs), b_li = al256(sizeof(int64_t) * n_jobs);
-    const size_t b_eo = al256(sizeof(uint64_t) * (n_jobs + 1)), b_j = al256(sizeof(nph_polya_job) * n_jobs);
     const size_t n_events_total = k.event_off.back();
     // the host needs the job lengths for the schedule and the scratch: the same values the kernel writes, from the host copies
     std::vector<nph_polya_job> hj(n_jobs);
@@ -473,20 +471,24 @@ extern "C" int nph_polya_after_load(nph_ctx* ctx, nph_polya_result* results_out,
     }
     ScratchPlan plan;
     NPH_TRY(plan_scratch(ctx, hj, &plan));
-    NPH_TRY(nph_reserve(ctx, ctx->d_polya, b_rj + b_tr + b_li + b_eo + b_j + run_scratch_bytes(n_jobs, plan)));
-    uint8_t* pb = ctx->d_polya.p;
-    nph_raw_job* d_rj = reinterpret_cast<nph_raw_job*>(pb); pb += b_rj;
-    nph_raw_range* d_tr = reinterpret_cast<nph_raw_range*>(pb); pb += b_tr;
-    int64_t* d_li = reinterpret_cast<int64_t*>(pb); pb += b_li;
-    uint64_t* d_eo = reinterpret_cast<uint64_t*>(pb); pb += b_eo;
-    nph_polya_job* d_j = reinterpret_cast<nph_polya_job*>(pb); pb += b_j;
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_rj, k.jobs.data(), sizeof(nph_raw_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_tr, ctx->h_last_trim.data(), sizeof(nph_raw_range) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_li, k.live_index.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_eo, k.event_off.data(), sizeof(uint64_t) * (n_jobs + 1), cudaMemcpyHostToDevice, ctx->stream));
+    struct { nph_raw_job* raw_jobs; nph_raw_range* trim; int64_t* live_index; uint64_t* event_off; nph_polya_job* jobs; } d{};
+    RunScratch rs;
+    auto layout = [&](NphCarve& a) {
+        d.raw_jobs = a.take<nph_raw_job>(n_jobs);
+        d.trim = a.take<nph_raw_range>(n_jobs);
+        d.live_index = a.take<int64_t>(n_jobs);
+        d.event_off = a.take<uint64_t>(n_jobs + 1);
+        d.jobs = a.take<nph_polya_job>(n_jobs);
+        rs = run_layout(a, n_jobs, plan);
+    };
+    NPH_TRY(nph_lay_out(ctx, ctx->d_polya, layout));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.raw_jobs, k.jobs.data(), sizeof(nph_raw_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.trim, ctx->h_last_trim.data(), sizeof(nph_raw_range) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.live_index, k.live_index.data(), sizeof(int64_t) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.event_off, k.event_off.data(), sizeof(uint64_t) * (n_jobs + 1), cudaMemcpyHostToDevice, ctx->stream));
     AfterLoadArgs al{};
-    al.raw_jobs = d_rj; al.trim = d_tr; al.live_index = d_li; al.event_off = d_eo; al.cal = k.d_cal; al.n_jobs = (uint32_t)n_jobs; al.jobs_out = d_j;
+    al.raw_jobs = d.raw_jobs; al.trim = d.trim; al.live_index = d.live_index; al.event_off = d.event_off; al.cal = k.d_cal; al.n_jobs = (uint32_t)n_jobs; al.jobs_out = d.jobs;
     after_load_jobs_kernel<<<(unsigned)((n_jobs + 127) / 128), 128, 0, ctx->stream>>>(al);
     NPH_CUDA(ctx, cudaGetLastError());
-    return run_polya(ctx, k.d_raw.p, k.n_samples_total, k.d_duration, n_events_total, k.d_b2e, k.n_ranks_total, d_j, hj, plan, pb, results_out);
+    return run_polya(ctx, k.d_raw.p, k.n_samples_total, k.d_duration, n_events_total, k.d_b2e, k.n_ranks_total, d.jobs, hj, plan, rs, results_out);
 }

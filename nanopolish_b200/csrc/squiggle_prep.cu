@@ -16,8 +16,6 @@
 #include <cstdlib>
 #include <cstring>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 namespace {
 
 constexpr unsigned kFull = 0xffffffffu;
@@ -363,21 +361,24 @@ __global__ void __launch_bounds__(kCalWarps * 32) recalibrate_kernel(const CalPa
     }
 }
 
-inline size_t al256(size_t v) { return (v + 255) / 256 * 256; }
-
 } // namespace
 
-size_t nph_trim_scratch_bytes(const nph_raw_read* reads, size_t n_reads, int32_t varseg_chunk)
+TrimScratch nph_trim_layout(NphCarve& a, const nph_raw_read* reads, size_t n_reads, int32_t varseg_chunk)
 {
     uint64_t n_chunks = 0;
     for (size_t i = 0; i < n_reads; ++i) n_chunks += reads[i].n_samples / (uint32_t)varseg_chunk;
-    return al256(sizeof(nph_raw_read) * n_reads) + al256(sizeof(uint64_t) * n_reads) + al256(sizeof(float) * (n_chunks + 1)) +
-           al256(sizeof(nph_raw_range) * n_reads);
+    TrimScratch s;
+    s.reads = a.take<nph_raw_read>(n_reads);
+    s.mad_off = a.take<uint64_t>(n_reads);
+    s.mad = a.take<float>(n_chunks + 1);
+    s.out = a.take<nph_raw_range>(n_reads);
+    return s;
 }
 
-// trim_and_segment_raw over reads whose samples are on the device; the ranges come back to the host (one sync).
+// trim_and_segment_raw over reads whose samples are on the device, in the scratch of nph_trim_layout; the ranges come
+// back to the host (one sync).
 int nph_trim_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_total, const nph_raw_read* reads, size_t n_reads,
-                    int32_t trim_start, int32_t trim_end, int32_t varseg_chunk, float varseg_thresh, uint8_t* scratch,
+                    int32_t trim_start, int32_t trim_end, int32_t varseg_chunk, float varseg_thresh, const TrimScratch& s,
                     nph_raw_range* ranges_out)
 {
     if (varseg_chunk < 2 || !(varseg_thresh >= 0.0f && varseg_thresh <= 1.0f) || trim_start < 0 || trim_end < 0) return NPH_ERR_INVALID;   // reference asserts
@@ -389,16 +390,12 @@ int nph_trim_device(nph_ctx* ctx, const float* d_raw, size_t n_samples_total, co
         mad_off[i] = n_chunks;
         n_chunks += reads[i].n_samples / (uint32_t)varseg_chunk;
     }
-    uint8_t* base = scratch;
     TrimParams p{};
-    nph_raw_read* d_reads = reinterpret_cast<nph_raw_read*>(base); base += al256(sizeof(nph_raw_read) * n_reads);
-    uint64_t* d_off = reinterpret_cast<uint64_t*>(base); base += al256(sizeof(uint64_t) * n_reads);
-    p.mad = reinterpret_cast<float*>(base); base += al256(sizeof(float) * (n_chunks + 1));
-    p.out = reinterpret_cast<nph_raw_range*>(base);
-    p.raw = d_raw; p.reads = d_reads; p.mad_off = d_off; p.n_reads = (uint32_t)n_reads;
+    p.mad = s.mad; p.out = s.out;
+    p.raw = d_raw; p.reads = s.reads; p.mad_off = s.mad_off; p.n_reads = (uint32_t)n_reads;
     p.trim_start = trim_start; p.trim_end = trim_end; p.chunk = varseg_chunk; p.perc = varseg_thresh;
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_reads, reads, sizeof(nph_raw_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_off, mad_off.data(), sizeof(uint64_t) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(s.reads, reads, sizeof(nph_raw_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(s.mad_off, mad_off.data(), sizeof(uint64_t) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
     trim_kernel<<<(unsigned)std::min<size_t>(n_reads, (size_t)ctx->sm_count * 8), kTrimThreads, 0, ctx->stream>>>(p);
     NPH_CUDA(ctx, cudaGetLastError());
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -428,14 +425,13 @@ extern "C" int nph_trim_raw_batch(nph_ctx* ctx, const float* raw, size_t n_sampl
     if (!raw || !reads || !ranges_out) return NPH_ERR_INVALID;
     if (varseg_chunk < 2) return NPH_ERR_INVALID;
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t b_raw = al256(sizeof(float) * n_samples_total);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, b_raw + nph_trim_scratch_bytes(reads, n_reads, varseg_chunk)));
-    ctx->abea_loaded = false;       // the arena is shared with the ABEA trace
-    float* d_raw = reinterpret_cast<float*>(ctx->d_abea_scratch.p);
+    float* d_raw = nullptr;
+    TrimScratch ts;
+    auto layout = [&](NphCarve& a) { d_raw = a.take<float>(n_samples_total); ts = nph_trim_layout(a, reads, n_reads, varseg_chunk); };
+    NPH_TRY(nph_borrow_arena(ctx, layout));
     NPH_CUDA(ctx, cudaMemcpyAsync(d_raw, raw, sizeof(float) * n_samples_total, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    NPH_TRY(nph_trim_device(ctx, d_raw, n_samples_total, reads, n_reads, trim_start, trim_end, varseg_chunk, varseg_thresh,
-                            ctx->d_abea_scratch.p + b_raw, ranges_out));
+    NPH_TRY(nph_trim_device(ctx, d_raw, n_samples_total, reads, n_reads, trim_start, trim_end, varseg_chunk, varseg_thresh, ts, ranges_out));
     ctx->last_launches = 1;
     ctx->timing_valid = true;
     return NPH_OK;
@@ -461,31 +457,28 @@ extern "C" int nph_recalibrate_batch(nph_ctx* ctx, const nph_read* reads, size_t
     for (size_t i = 0; i < n_ranks_total; ++i)
         if (kmer_ranks[i] >= n_states) return NPH_ERR_INVALID;
     NPH_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t b_ev = al256(sizeof(float) * n_events_total), b_reads = al256(sizeof(nph_read) * n_reads);
-    const size_t b_rk = al256(sizeof(uint32_t) * n_ranks_total), b_jobs = al256(sizeof(nph_abea_job) * n_jobs);
-    const size_t b_res = al256(sizeof(nph_abea_result) * n_jobs), b_pairs = al256(sizeof(nph_aligned_pair) * (pairs_total + 1));
-    const size_t b_b2e = al256(sizeof(nph_event_range) * n_ranks_total), b_cal = al256(sizeof(nph_calibration) * n_jobs);
-    NPH_TRY(nph_reserve(ctx, ctx->d_abea_scratch, b_ev + b_reads + b_rk + b_jobs + b_res + b_pairs + b_b2e + b_cal + 256));
-    ctx->abea_loaded = false;
-    uint8_t* base = ctx->d_abea_scratch.p;
     NphCalArgs a{};
-    float* d_ev = reinterpret_cast<float*>(base); base += b_ev;
-    nph_read* d_reads = reinterpret_cast<nph_read*>(base); base += b_reads;
-    uint32_t* d_rk = reinterpret_cast<uint32_t*>(base); base += b_rk;
-    nph_abea_job* d_jobs = reinterpret_cast<nph_abea_job*>(base); base += b_jobs;
-    nph_abea_result* d_res = reinterpret_cast<nph_abea_result*>(base); base += b_res;
-    nph_aligned_pair* d_pairs = reinterpret_cast<nph_aligned_pair*>(base); base += b_pairs;
-    a.b2e = reinterpret_cast<nph_event_range*>(base); base += b_b2e;
-    a.out = reinterpret_cast<nph_calibration*>(base); base += b_cal;
-    a.bad_input = reinterpret_cast<int*>(base);
-    a.ev_mean = d_ev; a.reads = d_reads; a.model_id = model_id; a.ranks = d_rk; a.jobs = d_jobs;
-    a.results = d_res; a.pairs = d_pairs; a.n_jobs = (uint32_t)n_jobs;
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_ev, ev_mean, sizeof(float) * n_events_total, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_reads, reads, sizeof(nph_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_rk, kmer_ranks, sizeof(uint32_t) * n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_jobs, jobs, sizeof(nph_abea_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    NPH_CUDA(ctx, cudaMemcpyAsync(d_res, results, sizeof(nph_abea_result) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
-    if (pairs_total) NPH_CUDA(ctx, cudaMemcpyAsync(d_pairs, pairs, sizeof(nph_aligned_pair) * pairs_total, cudaMemcpyHostToDevice, ctx->stream));
+    struct { float* ev; nph_read* reads; uint32_t* rk; nph_abea_job* jobs; nph_abea_result* res; nph_aligned_pair* pairs; } d{};
+    auto layout = [&](NphCarve& c) {
+        d.ev = c.take<float>(n_events_total);
+        d.reads = c.take<nph_read>(n_reads);
+        d.rk = c.take<uint32_t>(n_ranks_total);
+        d.jobs = c.take<nph_abea_job>(n_jobs);
+        d.res = c.take<nph_abea_result>(n_jobs);
+        d.pairs = c.take<nph_aligned_pair>(pairs_total + 1);
+        a.b2e = c.take<nph_event_range>(n_ranks_total);
+        a.out = c.take<nph_calibration>(n_jobs);
+        a.bad_input = c.take<int>(1);
+    };
+    NPH_TRY(nph_borrow_arena(ctx, layout));
+    a.ev_mean = d.ev; a.reads = d.reads; a.model_id = model_id; a.ranks = d.rk; a.jobs = d.jobs;
+    a.results = d.res; a.pairs = d.pairs; a.n_jobs = (uint32_t)n_jobs;
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.ev, ev_mean, sizeof(float) * n_events_total, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.reads, reads, sizeof(nph_read) * n_reads, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.rk, kmer_ranks, sizeof(uint32_t) * n_ranks_total, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.jobs, jobs, sizeof(nph_abea_job) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(d.res, results, sizeof(nph_abea_result) * n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    if (pairs_total) NPH_CUDA(ctx, cudaMemcpyAsync(d.pairs, pairs, sizeof(nph_aligned_pair) * pairs_total, cudaMemcpyHostToDevice, ctx->stream));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     NPH_TRY(nph_launch_recalibrate(ctx, a));
     NPH_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));

@@ -25,8 +25,6 @@
 #include <string>
 #include <vector>
 
-#define NPH_TRY(expr) do { int rc__ = (expr); if (rc__ != NPH_OK) return rc__; } while (0)
-
 int nph_launch_hmm_forward(nph_ctx* ctx, float* scores_dev);
 
 namespace {
@@ -521,22 +519,24 @@ extern "C" int nph_screen_fetch(nph_ctx* ctx, double* qualities_out, uint32_t* n
     NPH_TRY(make_dev(ctx, m.params, m.n_ref, d));
     const uint32_t n_pos = (uint32_t)m.n_pos;
     // outputs staged in the (now idle) score buffer region: 9 doubles + 1 uint32 per position
-    DevBuf<uint8_t>& scratch = ctx->d_prep;
     ctx->loaded_raw.valid = false;              // d_prep held the last load_from_raw batch's durations and map
+    struct { double* q; unsigned long long* r; uint32_t* n; } out{};
+    auto layout = [&](NphCarve& a) {
+        out.q = a.take<double>((size_t)NPH_SCREEN_SLOTS * n_pos);
+        out.r = a.take<unsigned long long>(n_pos);
+        out.n = a.take<uint32_t>(n_pos);
+    };
+    NPH_TRY(nph_lay_out(ctx, ctx->d_prep, layout));
     const size_t b_q = sizeof(double) * NPH_SCREEN_SLOTS * (size_t)n_pos, b_n = sizeof(uint32_t) * (size_t)n_pos;
     const size_t b_r = sizeof(unsigned long long) * (size_t)n_pos;
-    NPH_TRY(nph_reserve(ctx, scratch, b_q + b_r + b_n + 256));
-    double* d_q = reinterpret_cast<double*>(scratch.p);
-    unsigned long long* d_r = reinterpret_cast<unsigned long long*>(scratch.p + b_q);
-    uint32_t* d_n = reinterpret_cast<uint32_t*>(scratch.p + b_q + b_r);
-    var_output_kernel<<<(n_pos + kBlock - 1) / kBlock, kBlock, 0, ctx->stream>>>(d, reinterpret_cast<const PosState*>(m.d_state.p), m.d_pos_off.p, d_q, d_n, d_r);
+    var_output_kernel<<<(n_pos + kBlock - 1) / kBlock, kBlock, 0, ctx->stream>>>(d, reinterpret_cast<const PosState*>(m.d_state.p), m.d_pos_off.p, out.q, out.n, out.r);
     NPH_CUDA(ctx, cudaGetLastError());
-    NPH_CUDA(ctx, cudaMemcpyAsync(qualities_out, d_q, b_q, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(qualities_out, out.q, b_q, cudaMemcpyDeviceToHost, ctx->stream));
     std::vector<uint32_t> tmp;
     uint32_t* n_dst = n_reads_out;
     if (!n_dst) { tmp.resize(n_pos); n_dst = tmp.data(); }
-    NPH_CUDA(ctx, cudaMemcpyAsync(n_dst, d_n, b_n, cudaMemcpyDeviceToHost, ctx->stream));
-    if (reference_rows_out) NPH_CUDA(ctx, cudaMemcpyAsync(reference_rows_out, d_r, b_r, cudaMemcpyDeviceToHost, ctx->stream));
+    NPH_CUDA(ctx, cudaMemcpyAsync(n_dst, out.n, b_n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (reference_rows_out) NPH_CUDA(ctx, cudaMemcpyAsync(reference_rows_out, out.r, b_r, cudaMemcpyDeviceToHost, ctx->stream));
     NPH_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     // jobs a screening without early exit would have run: per position reads x (1 + candidates)
     uint64_t full = 0;
